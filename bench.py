@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # the B200 engine (torchrun for N > 1)
     python bench.py --impl reference --steps K --warmup W     # the reference's CPU arithmetic on host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also writes what the last timed step computed
+
+``--dump-outputs`` lets two builds be compared output for output: the inputs depend only on the arguments (seeded
+generators), and the files hold the level-0 result of the last timed step at k and at k = 16 (at most 36 MiB).
 
 A step is one ``ArrowDecompositionMPI.step()`` (forward exchange -> per-level arrow SpMM -> backward
 scatter-add) over the synthetic decomposition G2 of SURVEY.md 8d: 10M rows, width 10 000, two levels,
@@ -24,10 +28,13 @@ Prints ONE JSON line.
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -68,7 +75,15 @@ def parse():
     ap.add_argument("--no-k16", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the full-size parity property")
     ap.add_argument("--cpu-sample-blocks", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", type=str, default="", metavar="DIR",
+                    help="write the level-0 result of the last timed step (k and k = 16) as DIR/result_k<k>.npy, float32, "
+                         "rows in level-0 order: all rows, or a fixed seeded sample of them when the result is larger")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 engine computed (--impl b200)")
+    return a
 
 
 def measured_peak_gbs():
@@ -376,6 +391,32 @@ def time_steps(eng, ctx, barrier, steps, warmup, step_fn=None):
     return ctx.timer_ms(0) / steps
 
 
+DUMP_MAX_ROWS = 1 << 16          # 32 MB at k = 128
+DUMP_MAX_BYTES = 32 << 20        # per file: the k and k = 16 results stay below 64 MB together
+DUMP_SEED = 1009
+
+
+def dump_rows(n_rows, k):
+    """level-0 rows that ``--dump-outputs`` writes: every row, or a sorted sample drawn with a fixed seed, so that two
+    runs with the same arguments write the same rows"""
+    m = min(n_rows, DUMP_MAX_ROWS, DUMP_MAX_BYTES // (4 * k))
+    if m == n_rows:
+        return np.arange(n_rows)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n_rows, m, replace=False))
+
+
+def dump_result(directory, name, eng, host_out, row0, n_rows, comm):
+    """``directory/name.npy``: the level-0 result tile the last step left on the device (what ``B.result_tile()``
+    returns), rows of ``dump_rows`` in level-0 order.  Collective: every rank sends its rows of the sample, rank 0 writes."""
+    got = eng.result(0, host_out)
+    rows = dump_rows(n_rows, got.shape[1])
+    mine = rows[(rows >= row0) & (rows < row0 + got.shape[0])]
+    parts = sorted(comm.allgather((row0, got[mine - row0])), key=lambda p: p[0])
+    if comm.Get_rank() == 0:
+        os.makedirs(directory, exist_ok=True)
+        np.save(os.path.join(directory, name + ".npy"), np.concatenate([p for _, p in parts]))
+
+
 def level0_roofline(a, eng, k, world, dist, torch, steps):
     """the dominant launch alone; at N > 1 the slowest rank's launch against that rank's own algorithmic bytes"""
     peak, peak_src = measured_peak_gbs()
@@ -434,16 +475,18 @@ def run_b200(a):
 
     t_setup = time.time()
     comm = comm_mod.world_comm()
-    # the public path: files on disk -> load_decomposition_new -> initialize -> load blocks (every rank maps the same files)
+    # the public path: files on disk -> load_decomposition_new -> initialize -> load blocks (every rank maps the same files).
+    # The files go to a directory of this run, removed when it exits: the source tree may be read-only.
     tag = f"ba_{a.vertices}_{a.ba_m}" if a.workload == "ba" else f"{a.blocks}_{a.perm}"
-    base = os.path.join(ROOT, "tmp", f"bench_{tag}_{a.width}_{a.levels}")
+    files_dir = None
     if rank == 0:
-        done = base + ".complete"                           # written last: an interrupted generation is redone
-        if not os.path.exists(done):
-            dec0 = build_decomposition(a)
-            graphio.save_decomposition_new(dec0, base, a.width, block_diagonal=True)
-            del dec0
-            open(done, "w").close()
+        files_dir = tempfile.mkdtemp(prefix="arrow_b200_bench_")
+        atexit.register(shutil.rmtree, files_dir, ignore_errors=True)
+    base = os.path.join(comm.bcast(files_dir), f"bench_{tag}_{a.width}_{a.levels}")
+    if rank == 0:
+        dec0 = build_decomposition(a)
+        graphio.save_decomposition_new(dec0, base, a.width, block_diagonal=True)
+        del dec0
     comm.Barrier()
     arrow, eng, blocks = build_engine(a, comm, base, a.k, local_rank)
     dec = blocks.decomposition                 # memory-mapped level files (for the full-size property check)
@@ -475,10 +518,15 @@ def run_b200(a):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    launches0 = ctx.launch_count()
-    ms_step = time_steps(eng, ctx, barrier, a.steps, 0)
-    launches = ctx.launch_count() - launches0
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        launches0 = ctx.launch_count()
+        ms_step = time_steps(eng, ctx, barrier, a.steps, 0)
+        launches = ctx.launch_count() - launches0
+    finally:
+        clocks = sampler.stop() if rank == 0 else None      # no nvidia-smi left running if a step fails
+    n_rows = int(eng.n_blocks[0]) * a.width
+    if a.dump_outputs:
+        dump_result(a.dump_outputs, f"result_k{a.k}", eng, hostC.array, row0, n_rows, comm)
     ms_step = max_over_ranks(dist, torch, ms_step)
     flops = eng.flops_per_step()
     alg_bytes = eng.algorithmic_bytes_per_step()
@@ -573,6 +621,8 @@ def run_b200(a):
                 dist.barrier()
             eng16.sync()
         ms16 = max_over_ranks(dist, torch, time_steps(eng16, eng16.ctx, barrier16, a.steps, warm))
+        if a.dump_outputs:
+            dump_result(a.dump_outputs, "result_k16", eng16, c16.array, row0, n_rows, comm)
         roof16 = level0_roofline(a, eng16, 16, world, dist, torch, a.steps)
         ver16 = None if a.no_verify else verify_rank1_step(eng16, dec, a.width, row0, x16, c16, comm)
         k16 = {"metric": "iterated SpMM GFLOP/s (k=16)", "value": eng16.flops_per_step() / ms16 / 1e6, "unit": "GFLOP/s",

@@ -260,3 +260,45 @@ def test_bench_full_size_property_matches_the_protocol(levels, nested, tmp_path)
         assert "error" in bench.verify_rank1_step(None, dec, w, 0, Host(), Host(), SelfComm())
     else:
         assert "skipped" in v
+
+
+def test_bench_dump_outputs_fixed_sample_same_at_any_world_size(tmp_path):
+    """bench.py --dump-outputs: the level-0 result, whole when small, else a seeded row sample of bounded size; a world of
+    ranks writes the same file as one rank holding every row"""
+    import threading
+    import bench
+    from arrow_matrix_b200.comm import SelfComm, ThreadWorld
+
+    class Slice:                                         # a rank's engine: rows [r0, r1) of the level-0 result
+        def __init__(self, full, r0, r1):
+            self.tile = full[r0:r1]
+
+        def result(self, level, out):
+            out[:] = self.tile
+            return out
+
+    for n, k in ((300, 5), (100_000, 4), (70_000, 128)):
+        full = np.random.default_rng(n).random((n, k), dtype=np.float32)
+        rows = bench.dump_rows(n, k)
+        assert np.array_equal(rows, bench.dump_rows(n, k)) and np.all(np.diff(rows) > 0)
+        assert rows.size == n if n * k * 4 <= bench.DUMP_MAX_BYTES and n <= bench.DUMP_MAX_ROWS else rows.size < n
+        assert rows.size * k * 4 <= bench.DUMP_MAX_BYTES
+        one = tmp_path / f"one_{n}"
+        bench.dump_result(str(one), "result", Slice(full, 0, n), np.empty((n, k), np.float32), 0, n, SelfComm())
+        got = np.load(one / "result.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, full[rows])
+
+        bounds = [0, n // 3, n // 3 + 7, n]
+        world = ThreadWorld(3)
+        three = tmp_path / f"three_{n}"
+
+        def rank(r):
+            r0, r1 = bounds[r], bounds[r + 1]
+            bench.dump_result(str(three), "result", Slice(full, r0, r1), np.empty((r1 - r0, k), np.float32), r0, n,
+                              world.comm(r))
+        threads = [threading.Thread(target=rank, args=(r,)) for r in (2, 0, 1)]
+        for t in threads:
+            t.start()
+        for t in threads:
+            t.join()
+        assert np.array_equal(np.load(three / "result.npy"), got)
