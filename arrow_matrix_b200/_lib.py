@@ -19,6 +19,35 @@ LIB_PATH = os.path.join(_HERE, "libarrow_b200.so")
 ACCUMULATE = 1
 VARIANT_AUTO, VARIANT_DIRECT, VARIANT_SHFL, VARIANT_TMA, VARIANT_TILES = -1, 0, 1, 2, 3
 IPC_HANDLE_BYTES = 80
+DTYPE_CODES = {"float32": 0, "bfloat16": 1}      # ARROW_DTYPE_F32, ARROW_DTYPE_BF16
+
+
+def dtype_name(dtype) -> str:
+    """``"float32"`` or ``"bfloat16"`` for a dense-tile element type given as a name, a numpy dtype or a torch dtype;
+    ValueError for anything else (products and sums are fp32 either way)."""
+    if isinstance(dtype, str):
+        name = dtype
+    elif type(dtype).__module__ == "torch":
+        name = str(dtype).replace("torch.", "")
+    else:
+        try:
+            name = np.dtype(dtype).name
+        except TypeError:
+            name = str(dtype)
+    if name not in DTYPE_CODES:
+        raise ValueError(f"dense tiles hold float32 or bfloat16, not {dtype!r} (arithmetic is float32 in both)")
+    return name
+
+
+def to_bf16(X):
+    """Host rows as a contiguous CPU ``torch.bfloat16`` tensor: a bf16 tensor is taken as it is, anything else is
+    converted to float32 and rounded to nearest even (``Tensor.to(torch.bfloat16)``).  numpy has no bf16 type."""
+    import torch
+    if isinstance(X, torch.Tensor):
+        t = X if X.dtype == torch.bfloat16 else X.to(torch.float32).to(torch.bfloat16)
+    else:
+        t = torch.from_numpy(np.ascontiguousarray(X, dtype=np.float32)).to(torch.bfloat16)
+    return t.contiguous()
 
 EXPORTS = [
     "arrow_b200_abi_version", "arrow_ctx_create", "arrow_ctx_destroy", "arrow_last_error", "arrow_sync",
@@ -35,8 +64,9 @@ EXPORTS = [
     "arrow_ptrtable_upload", "arrow_ptrtable_free", "arrow_spmm_ex", "arrow_push_rows", "arrow_reduce_rows",
     "arrow_graph_begin", "arrow_graph_end", "arrow_graph_launch", "arrow_graph_free",
     "arrow_host_alloc_numa", "arrow_bind_thread_to_device_numa", "arrow_preload_kernels",
+    "arrow_dense_alloc_dtype", "arrow_dense_dtype", "arrow_dense_put", "arrow_dense_get",
 ]
-ABI_VERSION = 2          # ARROW_ABI_VERSION of include/arrow_b200.h this binding was written against
+ABI_VERSION = 3          # ARROW_ABI_VERSION of include/arrow_b200.h this binding was written against
 
 
 class ArrowError(RuntimeError):
@@ -128,6 +158,10 @@ def load_library(build_if_missing: bool = True) -> ctypes.CDLL:
         "arrow_host_alloc_numa": (c_int, [c_size_t, I, POINTER(P)]),
         "arrow_bind_thread_to_device_numa": (c_int, [I, pI, pI]),
         "arrow_preload_kernels": (c_int, [P, I]),
+        "arrow_dense_alloc_dtype": (c_int, [P, I64, I, I, pI]),
+        "arrow_dense_dtype": (c_int, [P, I, pI]),
+        "arrow_dense_put": (c_int, [P, I, I, I64, I64, P]),
+        "arrow_dense_get": (c_int, [P, I, I, I64, I64, P]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)          # AttributeError here = the .so does not export a declared symbol
@@ -172,6 +206,22 @@ class PinnedArray:
             self.close()
         except Exception:
             pass
+
+
+class PinnedTensor(PinnedArray):
+    """Page-locked host staging buffer exposed as a CPU torch tensor (``tensor``), for element types numpy lacks:
+    the bf16 rows ``ArrowEngine.stream_step`` moves for a bf16 engine."""
+
+    def __init__(self, shape, dtype=None, numa_device: Optional[int] = None):
+        import torch
+        dtype = torch.bfloat16 if dtype is None else dtype
+        itemsize = torch.empty(0, dtype=dtype).element_size()
+        super().__init__(shape, np.dtype(f"u{itemsize}"), numa_device)
+        self.tensor = torch.from_numpy(self.array).view(dtype)
+
+    def close(self):
+        self.tensor = None
+        super().close()
 
 
 def bind_thread_to_device_numa(device: int):
@@ -267,10 +317,15 @@ class Context:
         return RowMap(self, h.value, m.size, int(limit))
 
     # -- dense ------------------------------------------------------------------------------
-    def dense_alloc(self, rows: int, k: int) -> "Dense":
+    def dense_alloc(self, rows: int, k: int, dtype="float32") -> "Dense":
+        """zero-filled ``rows x k`` tile of ``dtype`` (float32 or bfloat16, see ``dtype_name``)"""
+        dtype = dtype_name(dtype)
         h = c_int()
-        self._check(self.lib.arrow_dense_alloc(self._h, int(rows), int(k), byref(h)))
-        return Dense(self, h.value, int(rows), int(k), owned=True)
+        if dtype == "float32":
+            self._check(self.lib.arrow_dense_alloc(self._h, int(rows), int(k), byref(h)))
+        else:
+            self._check(self.lib.arrow_dense_alloc_dtype(self._h, int(rows), int(k), DTYPE_CODES[dtype], byref(h)))
+        return Dense(self, h.value, int(rows), int(k), owned=True, dtype=dtype)
 
     def dense_wrap(self, device_ptr: int, rows: int, k: int) -> "Dense":
         h = c_int()
@@ -366,11 +421,20 @@ class Context:
     # -- copy lanes -------------------------------------------------------------------------
     LANE_MAIN, LANE_H2D, LANE_D2H = 0, 1, 2
 
-    def h2d_lane(self, lane: int, dst: "Dense", X: np.ndarray, row0: int = 0):
+    def h2d_lane(self, lane: int, dst: "Dense", X, row0: int = 0):
+        """``X``: float32 numpy rows for an fp32 tile, a contiguous CPU bf16 tensor for a bf16 tile"""
+        if dst.dtype == "bfloat16":
+            _check_bf16_host(X, dst.k)
+            self._check(self.lib.arrow_dense_put(self._h, lane, dst.h, int(row0), X.shape[0], c_void_p(X.data_ptr())))
+            return
         assert X.dtype == np.float32 and X.flags.c_contiguous and X.shape[1] == dst.k
         self._check(self.lib.arrow_dense_h2d_lane(self._h, lane, dst.h, int(row0), X.shape[0], _ptr(X)))
 
-    def d2h_lane(self, lane: int, src: "Dense", out: np.ndarray, row0: int = 0):
+    def d2h_lane(self, lane: int, src: "Dense", out, row0: int = 0):
+        if src.dtype == "bfloat16":
+            _check_bf16_host(out, src.k)
+            self._check(self.lib.arrow_dense_get(self._h, lane, src.h, int(row0), out.shape[0], c_void_p(out.data_ptr())))
+            return
         assert out.dtype == np.float32 and out.flags.c_contiguous and out.shape[1] == src.k
         self._check(self.lib.arrow_dense_d2h_lane(self._h, lane, src.h, int(row0), out.shape[0], _ptr(out)))
 
@@ -474,20 +538,46 @@ class PtrTable(_Handle):
         self._free("arrow_ptrtable_free")
 
 
-class Dense(_Handle):
-    def __init__(self, ctx, h, rows, k, owned):
-        super().__init__(ctx, h)
-        self.rows, self.k, self.owned = rows, k, owned
+def _check_bf16_host(t, k: int):
+    import torch
+    if not (isinstance(t, torch.Tensor) and t.dtype == torch.bfloat16 and t.device.type == "cpu" and t.is_contiguous()
+            and t.dim() == 2 and t.shape[1] == k):
+        raise ValueError(f"a bf16 tile moves rows as a contiguous CPU torch.bfloat16 tensor of [rows x {k}]")
 
-    def h2d(self, X: np.ndarray, row0: int = 0):
+
+class Dense(_Handle):
+    def __init__(self, ctx, h, rows, k, owned, dtype="float32"):
+        super().__init__(ctx, h)
+        self.rows, self.k, self.owned, self.dtype = rows, k, owned, dtype
+
+    def h2d(self, X, row0: int = 0):
+        """Upload rows starting at ``row0``.  A bf16 tile takes a CPU bf16 tensor, or float32 data that is rounded on the
+        host to nearest even (``to_bf16``)."""
+        if self.dtype == "bfloat16":
+            X = to_bf16(X)
+            _check_bf16_host(X, self.k)
+            self.ctx._check(self.ctx.lib.arrow_dense_put(self.ctx._h, 0, self.h, int(row0), X.shape[0], c_void_p(X.data_ptr())))
+            self._keep = X
+            return
         X = np.ascontiguousarray(X, dtype=np.float32)
         if X.ndim != 2 or X.shape[1] != self.k:
             raise ValueError(f"expected [rows x {self.k}] fp32, got {X.shape}")
         self.ctx._check(self.ctx.lib.arrow_dense_h2d(self.ctx._h, self.h, int(row0), X.shape[0], _ptr(X)))
         self._keep = X                  # async copy: keep the host array alive until the next sync
 
-    def d2h(self, out: Optional[np.ndarray] = None, row0: int = 0, rows: Optional[int] = None, sync: bool = True) -> np.ndarray:
+    def d2h(self, out=None, row0: int = 0, rows: Optional[int] = None, sync: bool = True):
+        """Download rows: a float32 numpy array, or a CPU bf16 tensor for a bf16 tile (``out`` of the same kind)."""
         rows = self.rows - row0 if rows is None else rows
+        if self.dtype == "bfloat16":
+            import torch
+            if out is None:
+                out = torch.empty((rows, self.k), dtype=torch.bfloat16)
+            _check_bf16_host(out, self.k)
+            assert out.shape[0] == rows
+            self.ctx._check(self.ctx.lib.arrow_dense_get(self.ctx._h, 0, self.h, int(row0), int(rows), c_void_p(out.data_ptr())))
+            if sync:
+                self.ctx.sync()
+            return out
         if out is None:
             out = np.empty((rows, self.k), dtype=np.float32)
         assert out.dtype == np.float32 and out.flags.c_contiguous and out.shape == (rows, self.k)

@@ -15,7 +15,7 @@ from typing import Optional
 import numpy as np
 
 from . import comm as comm_mod
-from . import graphio, synth, wb_logging
+from . import _lib, graphio, synth, wb_logging
 from .arrow_dec_mpi import ArrowDecompositionMPI
 
 
@@ -50,8 +50,10 @@ def bench_spmm(path: Optional[str], width: int, n_features: int, iterations: int
         name += "_Slim"
     wb_logging.wandb_init(comm, path, n_features, iterations, device, name, width, wandb_api_key)
 
+    # `datatype` is the element type of the feature tiles (float32 or bfloat16); matrix values load as float32 either way
+    feature_dtype = _lib.dtype_name(datatype)
     blocks, n_blocks, to_prev, to_next = ArrowDecompositionMPI.load_decomposition_new(
-        comm, path, width, blocked, datatype, slim=slim, use_npy=npy_format)
+        comm, path, width, blocked, np.float32, slim=slim, use_npy=npy_format)
     if blocks is not None and verbose:
         print("RANK loaded decomposition", rank, n_blocks, flush=True)
     comm.Barrier()
@@ -68,13 +70,13 @@ def bench_spmm(path: Optional[str], width: int, n_features: int, iterations: int
         wb_logging.log({"actual_ranks": comm.Get_size()})
         tic = time.perf_counter()
         arrow.B.load_sparse_matrix_from_blocks(blocks)
-        arrow.B.zero_rhs(width, n_features)
+        arrow.B.zero_rhs(width, n_features, dtype=feature_dtype)
         arrow.synchronize()
         comm.Barrier()
         wb_logging.log({"init_time": time.perf_counter() - tic})
         rows_local = arrow._engine.local_rows_of(0)
         for i in range(iterations):
-            X_p0 = 2 * rng.random((rows_local, n_features), dtype=datatype) - 1      # arrow_bench.py:115
+            X_p0 = 2 * rng.random((rows_local, n_features), dtype=np.float32) - 1    # arrow_bench.py:115 (bf16: rounded on upload)
             arrow.B.set_features(X_p0)
             comm.Barrier()
             fail = False

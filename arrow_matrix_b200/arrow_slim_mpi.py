@@ -12,6 +12,7 @@ from typing import Optional
 
 import numpy as np
 
+from . import _lib
 from .arrow_matrix import ArrowMatrix
 
 
@@ -39,8 +40,9 @@ class ArrowSlimMPI(ArrowMatrix):
         _require_gpu(device)
         self._engine.spmm_level(self._level)
 
-    def result_tile(self, out: Optional[np.ndarray] = None) -> np.ndarray:
-        """Host copy of this process's result rows; pass a (pinned) ``out`` array to avoid an allocation per call."""
+    def result_tile(self, out=None):
+        """Host copy of this process's result rows (a CPU bf16 tensor after ``zero_rhs(dtype=torch.bfloat16)``); pass a
+        (pinned) ``out`` of the same kind to avoid an allocation per call."""
         return self._engine.result(self._level, out)
 
     @property
@@ -51,13 +53,18 @@ class ArrowSlimMPI(ArrowMatrix):
     def feature_tile(self) -> np.ndarray:
         return self._engine.features(self._level)
 
-    def set_features(self, X: np.ndarray) -> None:
+    def set_features(self, X) -> None:
         """Upload this process's feature rows (level 0).  The reference keeps a reference to ``X``
-        (arrow_slim_mpi.py:285-293); here the rows are copied to the device at call time."""
+        (arrow_slim_mpi.py:285-293); here the rows are copied to the device at call time.  With bf16 tiles ``X`` may be
+        a CPU bf16 tensor; float32 rows are rounded to nearest even."""
         assert X is not None
         if self._level != 0:
             raise ValueError("features enter at level 0; deeper levels receive them through the exchange")
-        self._engine.set_features(np.ascontiguousarray(X, dtype=np.float32))
+        eng = self._engine
+        if getattr(eng, "dtype", "float32") == "bfloat16":
+            eng.set_features(X)
+        else:
+            eng.set_features(np.ascontiguousarray(X, dtype=np.float32))
 
     def load_sparse_matrix_from_blocks(self, blocks) -> None:
         """``blocks`` is what ``ArrowDecompositionMPI.load_decomposition_new`` returned."""
@@ -65,12 +72,23 @@ class ArrowSlimMPI(ArrowMatrix):
         self.tiles_per_side = self._engine.n_blocks[self._level]
 
     def zero_rhs(self, number_of_rows_per_rank: int, number_of_columns: int, dtype=np.float32) -> None:
+        """Zero the tiles (arrow_slim_mpi.py:354-394).  ``dtype`` is the element type of the feature and result tiles:
+        float32 (default) or bfloat16 (``torch.bfloat16`` / ``"bfloat16"``: half the bytes per row, arithmetic still
+        float32, one GPU only); switching re-allocates the tiles."""
         assert number_of_rows_per_rank >= 1 and number_of_columns >= 1
-        if np.dtype(dtype) != np.float32:
-            raise ValueError("the B200 path computes in float32 (like the reference's benchmark, arrow_bench.py:21)")
+        try:
+            dtype = _lib.dtype_name(dtype)
+        except ValueError:
+            raise ValueError(f"the B200 path stores features as float32 or bfloat16 and computes in float32 "
+                             f"(like the reference's benchmark, arrow_bench.py:21), not {dtype!r}") from None
+        if dtype == "bfloat16" and self.comm.Get_size() > 1:
+            raise NotImplementedError("bf16 feature tiles run on one GPU; the N-GPU engine in bf16 (sharded fused step, "
+                                      "exchange protocol, NCCL) is a follow-up -- use float32 with more than one rank")
         eng = self._engine
         if number_of_columns != eng.k or number_of_rows_per_rank != eng.width:
             raise ValueError(f"engine was initialised for width={eng.width}, k={eng.k}")
+        if hasattr(eng, "set_dtype"):
+            eng.set_dtype(dtype)
         eng.zero_rhs()
 
     def is_column_rank(self) -> bool:

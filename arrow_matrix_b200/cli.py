@@ -34,6 +34,8 @@ def main(argv=None) -> None:
                         help='Reference rank layout selector; both layouts map to the same GPU kernels.')
     parser.add_argument('-n', '--npy', type=str2bool, nargs="?", default=True,
                         help='If true, the decomposition is loaded from the indices / indptr files.')
+    parser.add_argument('--dtype', choices=('float32', 'bfloat16'), default='float32',
+                        help='Element type of the feature and result tiles (one GPU for bfloat16); arithmetic is float32.')
     args = vars(parser.parse_args(argv))
     from . import comm as comm_mod
     comm_mod.init_from_env()                    # torchrun --nproc-per-node N: one process per GPU
@@ -41,7 +43,7 @@ def main(argv=None) -> None:
         print(str(args), flush=True)
     arrow_bench.bench_spmm(args['path'], args['width'], args['features'], args['iterations'], args['blocked'],
                            args['device'], args['ranksperside'], args['ba_neighbors'], None,
-                           slim=args['slim'], npy_format=args['npy'])
+                           datatype=args['dtype'], slim=args['slim'], npy_format=args['npy'])
 
 
 if __name__ == '__main__':

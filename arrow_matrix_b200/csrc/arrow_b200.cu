@@ -8,10 +8,12 @@
 //   remapped columns    arrow_dec_mpi.py:526,544  (`feature_tile()[perm]` + `C_i[perm] = recvbuf`)
 //   k_gather_rows*      the same two exchanges as standalone (un-fused / cross-GPU) steps
 //
-// Layout: CSR = int32 indptr (rebased to 0) / int32 indices / fp32 values; dense tiles row-major fp32.
+// Layout: CSR = int32 indptr (rebased to 0) / int32 indices / fp32 values; dense tiles row-major fp32 or bf16 (one-GPU
+// launches; fp32 arithmetic, each stored bf16 row rounded once to nearest even).
 // All kernels are HBM/L2-bandwidth bound gathers (about 2 FLOP/B): no tensor cores on purpose.
 #include "../../include/arrow_b200.h"
 
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <ctype.h>
 #include <dlfcn.h>
@@ -37,13 +39,16 @@
 namespace {
 
 struct DenseBuf {
-    float *p = nullptr;
+    float *p = nullptr;               // ARROW_DTYPE_BF16: the bits of bf16 elements (use esize(), never p + i for an offset)
     int64_t rows = 0;
     int k = 0;
+    int dtype = ARROW_DTYPE_F32;
     bool owned = false;
     bool ipc = false;
     void *ipc_base = nullptr;
     bool live = false;
+    size_t esize() const { return dtype == ARROW_DTYPE_BF16 ? 2 : 4; }
+    char *row(int64_t r) const { return reinterpret_cast<char *>(p) + (size_t)r * k * esize(); }
 };
 
 struct LongTask {      // one segment of a long row
@@ -208,6 +213,12 @@ IdxMap *get_map(arrow_ctx *ctx, int h) {
     return &ctx->maps[h];
 }
 
+// the entry points of the N-GPU path and the float * copies take fp32 tiles only
+#define REQUIRE_F32(ctx, d, what)                                                                              \
+    do {                                                                                                       \
+        if ((d)->dtype != ARROW_DTYPE_F32) return fail((ctx), ARROW_ERR_ARG, "%s needs an fp32 tile (this one is bf16)", (what)); \
+    } while (0)
+
 inline int ceil_div_i64(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
 // frees whatever device arrays the block owns (cudaFree waits for the device, so no launch can still read them)
@@ -244,16 +255,76 @@ __device__ __forceinline__ void f4_add(float4 &acc, const float4 &x) {
     acc.x += x.x; acc.y += x.y; acc.z += x.z; acc.w += x.w;
 }
 
+typedef __nv_bfloat16 bf16;
+
+// Element type of the dense tiles of a launch.  The vector kernels move rows as 16-byte vectors held in float4
+// registers as raw bits (4 fp32 or 8 bf16 values) and accumulate one vector in an `Acc` of fp32; `pack` is the one
+// rounding of a stored row.  Scalar kernels use to_f / from_f.
+template <typename T>
+struct Elt;
+template <>
+struct Elt<float> {
+    static constexpr int PER_VEC = 4;
+    using Acc = float4;
+    static __device__ __forceinline__ Acc zero() { return f4_zero(); }
+    static __device__ __forceinline__ Acc widen(const float4 &x) { return x; }
+    static __device__ __forceinline__ void fma(Acc &acc, float a, const float4 &x) { f4_fma(acc, a, x); }
+    static __device__ __forceinline__ void add(Acc &acc, const float4 &x) { f4_add(acc, x); }
+    static __device__ __forceinline__ float4 pack(const Acc &acc) { return acc; }
+    static __device__ __forceinline__ float to_f(float x) { return x; }
+    static __device__ __forceinline__ float from_f(float x) { return x; }
+};
+template <>
+struct Elt<bf16> {
+    static constexpr int PER_VEC = 8;
+    struct Acc { float4 lo, hi; };                  // elements 0..3, 4..7 of the vector
+    // bf16 -> fp32 is exact: the element becomes the upper half of an fp32 word (a shift or a mask, no F2F).  Element
+    // 2i is the low half of word i (little endian), element 2i+1 the high half.
+    static __device__ __forceinline__ float lo(float w) { return __uint_as_float(__float_as_uint(w) << 16); }
+    static __device__ __forceinline__ float hi(float w) { return __uint_as_float(__float_as_uint(w) & 0xffff0000u); }
+    static __device__ __forceinline__ Acc zero() { return Acc{f4_zero(), f4_zero()}; }
+    static __device__ __forceinline__ Acc widen(const float4 &x) {
+        return Acc{make_float4(lo(x.x), hi(x.x), lo(x.y), hi(x.y)), make_float4(lo(x.z), hi(x.z), lo(x.w), hi(x.w))};
+    }
+    static __device__ __forceinline__ void fma(Acc &acc, float a, const float4 &x) {
+        acc.lo.x = fmaf(a, lo(x.x), acc.lo.x);
+        acc.lo.y = fmaf(a, hi(x.x), acc.lo.y);
+        acc.lo.z = fmaf(a, lo(x.y), acc.lo.z);
+        acc.lo.w = fmaf(a, hi(x.y), acc.lo.w);
+        acc.hi.x = fmaf(a, lo(x.z), acc.hi.x);
+        acc.hi.y = fmaf(a, hi(x.z), acc.hi.y);
+        acc.hi.z = fmaf(a, lo(x.w), acc.hi.z);
+        acc.hi.w = fmaf(a, hi(x.w), acc.hi.w);
+    }
+    static __device__ __forceinline__ void add(Acc &acc, const float4 &x) {
+        const Acc w = widen(x);
+        f4_add(acc.lo, w.lo);
+        f4_add(acc.hi, w.hi);
+    }
+    static __device__ __forceinline__ float pack2(float e0, float e1) {      // round-to-nearest-even, e0 in the low half
+        uint32_t r;
+        asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(e1), "f"(e0));
+        return __uint_as_float(r);
+    }
+    static __device__ __forceinline__ float4 pack(const Acc &a) {
+        return make_float4(pack2(a.lo.x, a.lo.y), pack2(a.lo.z, a.lo.w), pack2(a.hi.x, a.hi.y), pack2(a.hi.z, a.hi.w));
+    }
+    static __device__ __forceinline__ float to_f(bf16 x) { return __bfloat162float(x); }
+    static __device__ __forceinline__ bf16 from_f(float x) { return __float2bfloat16_rn(x); }
+};
+template <typename T>
+constexpr bool is_bf16() { return std::is_same<T, bf16>::value; }
+
 struct SpmmArgs {
     const int *__restrict__ indptr;
     const int *__restrict__ indices;
     const float *__restrict__ vals;
-    const float *__restrict__ X;
+    const float *__restrict__ X;      // dense tiles (X, C, X2, add_src) hold the launch's element type T (Elt<T>)
     float *__restrict__ C;
     const int *__restrict__ rowmap;   // nullptr: identity
     long long n_rows;
     int k;                            // feature columns
-    int k4;                           // k / 4 (vector kernels)
+    int k4;                           // 16-byte vectors per row: k / Elt<T>::PER_VEC (vector kernels)
     int long_threshold;               // rows with more entries are left to the long-row kernels
     const float *__restrict__ add_src;   // optional addend: C[r] = sum + add_src[add_map[r]] (add_map[r] >= 0), else nullptr
     const int *__restrict__ add_map;
@@ -261,12 +332,6 @@ struct SpmmArgs {
     int x_split;
     float *const *__restrict__ out_ptr;  // optional destination pointer per row (nullptr entry = row dropped); overrides C / rowmap
 };
-
-// row `c` of the (possibly two-part) X operand
-__device__ __forceinline__ const float *x_row_ptr(const SpmmArgs &a, int c) {
-    if (a.X2 != nullptr && c >= a.x_split) return a.X2 + (long long)(c - a.x_split) * a.k;
-    return a.X + (long long)c * a.k;
-}
 
 // ------------------------------------------------------------------------------------------------
 // variant 0: a group of G lanes owns one row; every lane of the group reads the same index/value
@@ -684,8 +749,9 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *gptr, uint32_t byte
 // launch (scattered first-touch gathers, latency bound) measured 2.2-2.6 ms against 1.8 ms for this code on the same GPU
 // (profiles/r02_kernel_sweep.md, section 5); ARROW_OPT_TILE_KERNEL switches between the two.
 // ------------------------------------------------------------------------------------------------
-template <int G, int VPL, bool ROWMAP, bool ACC, int TR, int TN>
+template <typename T, int G, int VPL, bool ROWMAP, bool ACC, int TR, int TN>
 __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
+    using E = Elt<T>;
     constexpr int TILE_PTR_WORDS = TileCfg<TR, TN>::PTR_WORDS;
     constexpr int TILE_NNZ_WORDS = TileCfg<TR, TN>::NNZ_WORDS;
     constexpr int TILE_STAGE_WORDS = TileCfg<TR, TN>::STAGE_WORDS;
@@ -785,11 +851,11 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
             }
             // accumulate mode: the old C row is read FIRST so that its latency hides behind the gathers (only this
             // group ever touches the row: the row maps are injective)
-            float4 acc[VPL];
+            typename E::Acc acc[VPL];
             float4 *cr = Cl + orow * k4;
 #pragma unroll
             for (int i = 0; i < VPL; ++i)
-                acc[i] = (ACC && gl + i * G < k4) ? ld_f4_hint(cr + i * G, pol_stream) : f4_zero();
+                acc[i] = (ACC && gl + i * G < k4) ? E::widen(ld_f4_hint(cr + i * G, pol_stream)) : E::zero();
             if (a.add_map != nullptr) {
                 // epilogue gather-add, issued first so its latency hides behind the gathers: the backward exchange
                 // C_{j-1}[to_prev[r]] += C_j[r] (arrow_dec_mpi.py:437) seen from the receiving row
@@ -798,7 +864,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
                     const float4 *ar = reinterpret_cast<const float4 *>(a.add_src) + (long long)am * k4 + gl;
 #pragma unroll
                     for (int i = 0; i < VPL; ++i)
-                        if (gl + i * G < k4) f4_add(acc[i], ld_f4_hint(ar + i * G, pol_stream));
+                        if (gl + i * G < k4) E::add(acc[i], ld_f4_hint(ar + i * G, pol_stream));
                 }
             }
             int p = s;
@@ -824,7 +890,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
 #pragma unroll
                     for (int u = 0; u < N; ++u)
 #pragma unroll
-                        for (int i = 0; i < VPL; ++i) f4_fma(acc[i], v[u], x[u][i]);
+                        for (int i = 0; i < VPL; ++i) E::fma(acc[i], v[u], x[u][i]);
                     p += N;
                 };
                 while (p + UNROLL <= e) batch(std::integral_constant<int, UNROLL>{});
@@ -853,11 +919,11 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
 #pragma unroll
                 for (int u = 0; u < TAIL; ++u)
 #pragma unroll
-                    for (int i = 0; i < VPL; ++i) f4_fma(acc[i], v[u], x[u][i]);
+                    for (int i = 0; i < VPL; ++i) E::fma(acc[i], v[u], x[u][i]);
             }
 #pragma unroll
             for (int i = 0; i < VPL; ++i)
-                if (gl + i * G < k4) st_f4_hint(cr + i * G, acc[i], pol_stream);
+                if (gl + i * G < k4) st_f4_hint(cr + i * G, E::pack(acc[i]), pol_stream);
         }
         __syncthreads();            // stage `st` may be refilled by the next iteration's prefetch
         tile = s_next[st];
@@ -868,8 +934,9 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
 // half the batch size per row: the gathers of both rows are issued before either row's FMAs.  Same registers, but the
 // short tail batch of one row (a 10-entry row is 8 + 2 gathers: the second round trip keeps 2 of 8 slots busy) overlaps
 // the other row's -- narrow feature tiles (k <= 32) are bound by gathers in flight, not by bandwidth.
-template <int G, int VPL, int OUT, bool ACC, int TR, int TN, int RPG, int MINB, bool DUALX>
+template <typename T, int G, int VPL, int OUT, bool ACC, int TR, int TN, int RPG, int MINB, bool DUALX>
 __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
+    using E = Elt<T>;
     constexpr int TILE_PTR_WORDS = TileCfg<TR, TN>::PTR_WORDS;
     constexpr int TILE_NNZ_WORDS = TileCfg<TR, TN>::NNZ_WORDS;
     constexpr int TILE_STAGE_WORDS = TileCfg<TR, TN>::STAGE_WORDS;
@@ -953,7 +1020,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
             // Bulk L2 prefetch of this tile's X rows (one cp.async.bulk.prefetch.L2 per row, issued by the TMA unit: no
             // registers, no LSU wavefronts).  Measured in round 2 (profiles/r02_kernel_sweep.md): a LOSS at every k -- the
             // request rate of the unit, not DRAM latency, becomes the bound.  Off by default; kept as the A/B switch.
-            const uint32_t row_bytes = (uint32_t)a.k * 4u;
+            const uint32_t row_bytes = (uint32_t)a.k * (uint32_t)sizeof(T);
             for (int q = d.z + (int)threadIdx.x; q < d.w; q += TILE_THREADS) {
                 const int cq = s_idx[q];
                 if (cq >= 0) bulk_prefetch_l2(xrow(cq) - gl, row_bytes);
@@ -966,7 +1033,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
             int p[NR], e[NR];
             bool live[NR];
             float4 *cr[NR];
-            float4 acc[NR][VPL];
+            typename E::Acc acc[NR][VPL];
 #pragma unroll
             for (int r = 0; r < NR; ++r) {
                 const int lr = lr0 + r * ROWS_PER_PASS;
@@ -998,7 +1065,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
                 // group ever touches the row: the row maps are injective)
 #pragma unroll
                 for (int i = 0; i < VPL; ++i)
-                    acc[r][i] = (ACC && live[r] && gl + i * G < k4) ? ld_f4_hint(cr[r] + i * G, pol_stream) : f4_zero();
+                    acc[r][i] = (ACC && live[r] && gl + i * G < k4) ? E::widen(ld_f4_hint(cr[r] + i * G, pol_stream)) : E::zero();
                 if (a.add_map != nullptr && live[r]) {
                     // epilogue gather-add, issued first so its latency hides behind the gathers: the backward exchange
                     // C_{j-1}[to_prev[r]] += C_j[r] (arrow_dec_mpi.py:437) seen from the receiving row
@@ -1007,7 +1074,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
                         const float4 *ar = reinterpret_cast<const float4 *>(a.add_src) + (long long)am * k4 + gl;
 #pragma unroll
                         for (int i = 0; i < VPL; ++i)
-                            if (gl + i * G < k4) f4_add(acc[r][i], ld_f4_hint(ar + i * G, pol_stream));
+                            if (gl + i * G < k4) E::add(acc[r][i], ld_f4_hint(ar + i * G, pol_stream));
                     }
                 }
             }
@@ -1030,7 +1097,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
 #pragma unroll
                         for (int u = 0; u < N; ++u)
 #pragma unroll
-                            for (int i = 0; i < VPL; ++i) f4_fma(acc[0][i], v[u], x[u][i]);
+                            for (int i = 0; i < VPL; ++i) E::fma(acc[0][i], v[u], x[u][i]);
                         p[0] += N;
                     };
                     while (p[0] + UNROLL <= e[0]) batch(std::integral_constant<int, UNROLL>{});
@@ -1056,7 +1123,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
                             for (int u = 0; u < UNROLL; ++u) {
                                 const float v = s_val[p[r] + u];
 #pragma unroll
-                                for (int i = 0; i < VPL; ++i) f4_fma(acc[r][i], v, x[r][u][i]);
+                                for (int i = 0; i < VPL; ++i) E::fma(acc[r][i], v, x[r][u][i]);
                             }
                             p[r] += UNROLL;
                         }
@@ -1079,7 +1146,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
                             for (int u = 0; u < UNROLL; ++u) {
                                 const float v = (p[r] + u < e[r]) ? s_val[p[r] + u] : 0.f;
 #pragma unroll
-                                for (int i = 0; i < VPL; ++i) f4_fma(acc[r][i], v, x[r][u][i]);
+                                for (int i = 0; i < VPL; ++i) E::fma(acc[r][i], v, x[r][u][i]);
                             }
                             p[r] = min(p[r] + UNROLL, e[r]);
                         }
@@ -1109,16 +1176,16 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
 #pragma unroll
                     for (int u = 0; u < TAIL; ++u)
 #pragma unroll
-                        for (int i = 0; i < VPL; ++i) f4_fma(acc[r][i], v[u], x[u][i]);
+                        for (int i = 0; i < VPL; ++i) E::fma(acc[r][i], v[u], x[u][i]);
                 }
                 if (live[r]) {
 #pragma unroll
                     for (int i = 0; i < VPL; ++i) {
                         if (gl + i * G < k4) {
                             if constexpr (OUT == OUT_ROWPTR) {
-                                *(cr[r] + i * G) = acc[r][i];       // may be a peer GPU's memory (NVLink store): no L2 policy
+                                *(cr[r] + i * G) = E::pack(acc[r][i]);       // may be a peer GPU's memory (NVLink store): no L2 policy
                             } else {
-                                st_f4_hint(cr[r] + i * G, acc[r][i], pol_stream);
+                                st_f4_hint(cr[r] + i * G, E::pack(acc[r][i]), pol_stream);
                             }
                         }
                     }
@@ -1146,10 +1213,14 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// generic k (not a multiple of 4): warp per row, lanes over columns, scalar accesses.
+// generic k (not a multiple of one 16-byte vector: 4 fp32 / 8 bf16): warp per row, lanes over columns, scalar accesses.
 // ------------------------------------------------------------------------------------------------
-template <bool ROWMAP, bool ACC>
+template <typename T, bool ROWMAP, bool ACC>
 __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
+    using E = Elt<T>;
+    const T *__restrict__ X = reinterpret_cast<const T *>(a.X);
+    const T *__restrict__ X2 = reinterpret_cast<const T *>(a.X2);
+    const T *__restrict__ add_src = reinterpret_cast<const T *>(a.add_src);
     const int lane = threadIdx.x & 31;
     const long long warps_total = (long long)gridDim.x * (blockDim.x >> 5);
     const long long warp_id = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -1162,9 +1233,9 @@ __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
             orow = __ldg(a.rowmap + row);
             if (orow < 0) continue;
         }
-        float *crow = a.C + orow * a.k;
+        T *crow = reinterpret_cast<T *>(a.C) + orow * a.k;
         if (a.out_ptr != nullptr) {
-            crow = a.out_ptr[row];
+            crow = reinterpret_cast<T *>(a.out_ptr[row]);
             if (crow == nullptr) continue;
         }
         for (int c0 = 0; c0 < a.k; c0 += 128) {
@@ -1173,11 +1244,11 @@ __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
                 const int c = __ldg(a.indices + p);
                 const float v = __ldg(a.vals + p);
                 if (c < 0) continue;
-                const float *xr = x_row_ptr(a, c);
+                const T *xr = (X2 != nullptr && c >= a.x_split) ? X2 + (long long)(c - a.x_split) * a.k : X + (long long)c * a.k;
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
                     const int col = c0 + lane + 32 * i;
-                    if (col < a.k) acc[i] = fmaf(v, __ldg(xr + col), acc[i]);
+                    if (col < a.k) acc[i] = fmaf(v, E::to_f(__ldg(xr + col)), acc[i]);
                 }
             }
             const int am = (a.add_map != nullptr) ? __ldg(a.add_map + row) : -1;
@@ -1185,10 +1256,10 @@ __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
             for (int i = 0; i < 4; ++i) {
                 const int col = c0 + lane + 32 * i;
                 if (col < a.k) {
-                    float *dst = crow + col;
-                    float r = ACC ? (*dst + acc[i]) : acc[i];
-                    if (am >= 0) r += a.add_src[(long long)am * a.k + col];
-                    *dst = r;
+                    T *dst = crow + col;
+                    float r = ACC ? (E::to_f(*dst) + acc[i]) : acc[i];
+                    if (am >= 0) r += E::to_f(add_src[(long long)am * a.k + col]);
+                    *dst = E::from_f(r);
                 }
             }
         }
@@ -1203,14 +1274,17 @@ struct LongArgs {
     const LongTask *__restrict__ tasks;
     const int *__restrict__ indices;
     const float *__restrict__ vals;
-    const float *__restrict__ X;
-    float *__restrict__ scratch;      // [slot][k]
+    const float *__restrict__ X;      // element type T of k_spmm_long_partial<T>
+    float *__restrict__ scratch;      // [slot][k], fp32 whatever T
     int k;
     const float *__restrict__ X2;     // second X base (see SpmmArgs)
     int x_split;
 };
 
+template <typename T>
 __global__ void __launch_bounds__(256) k_spmm_long_partial(LongArgs a) {
+    const T *__restrict__ X = reinterpret_cast<const T *>(a.X);
+    const T *__restrict__ X2 = reinterpret_cast<const T *>(a.X2);
     extern __shared__ float red[];    // [warps][k]
     const LongTask t = a.tasks[blockIdx.x];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
@@ -1220,11 +1294,11 @@ __global__ void __launch_bounds__(256) k_spmm_long_partial(LongArgs a) {
             const int c = __ldg(a.indices + p);
             const float v = __ldg(a.vals + p);
             if (c < 0) continue;
-            const float *xr = (a.X2 != nullptr && c >= a.x_split) ? a.X2 + (long long)(c - a.x_split) * a.k : a.X + (long long)c * a.k;
+            const T *xr = (X2 != nullptr && c >= a.x_split) ? X2 + (long long)(c - a.x_split) * a.k : X + (long long)c * a.k;
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
                 const int col = c0 + lane + 32 * i;
-                if (col < a.k) acc[i] = fmaf(v, __ldg(xr + col), acc[i]);
+                if (col < a.k) acc[i] = fmaf(v, Elt<T>::to_f(__ldg(xr + col)), acc[i]);
             }
         }
 #pragma unroll
@@ -1241,22 +1315,23 @@ __global__ void __launch_bounds__(256) k_spmm_long_partial(LongArgs a) {
     }
 }
 
-template <bool ROWMAP, bool ACC>
+template <typename T, bool ROWMAP, bool ACC>
 __global__ void __launch_bounds__(128) k_spmm_long_reduce(const int *__restrict__ long_rows,
                                                           const int *__restrict__ long_first,
                                                           const float *__restrict__ scratch,
-                                                          float *__restrict__ C, const int *__restrict__ rowmap, int k,
-                                                          const float *__restrict__ add_src, const int *__restrict__ add_map,
+                                                          T *__restrict__ C, const int *__restrict__ rowmap, int k,
+                                                          const T *__restrict__ add_src, const int *__restrict__ add_map,
                                                           float *const *__restrict__ out_ptr) {
+    using E = Elt<T>;
     const int r = long_rows[blockIdx.x];
     long long orow = r;
     if (ROWMAP) {
         orow = rowmap[r];
         if (orow < 0) return;
     }
-    float *crow = C + orow * k;
+    T *crow = C + orow * k;
     if (out_ptr != nullptr) {
-        crow = out_ptr[r];
+        crow = reinterpret_cast<T *>(out_ptr[r]);
         if (crow == nullptr) return;
     }
     const int s0 = long_first[blockIdx.x], s1 = long_first[blockIdx.x + 1];
@@ -1265,10 +1340,10 @@ __global__ void __launch_bounds__(128) k_spmm_long_reduce(const int *__restrict_
         for (int s = s0; s < s1; ++s) sum += scratch[(long long)s * k + col];
         if (add_map != nullptr) {
             const int am = add_map[r];
-            if (am >= 0) sum += add_src[(long long)am * k + col];
+            if (am >= 0) sum += E::to_f(add_src[(long long)am * k + col]);
         }
-        float *dst = crow + col;
-        *dst = ACC ? (*dst + sum) : sum;
+        T *dst = crow + col;
+        *dst = E::from_f(ACC ? (E::to_f(*dst) + sum) : sum);
     }
 }
 
@@ -1285,7 +1360,20 @@ struct MultiSrc {
 // A group of G lanes moves one row (VPR vectors of VT); rows are taken warp-strided so that a warp's
 // destination rows are consecutive (coalesced stores) while the sources are wherever the map points --
 // local HBM, or a peer GPU's memory over NVLink when MULTI.
-template <typename VT, int G, bool ACC, bool MULTI>
+// dst row (+)= src row for one vector (4 fp32 / 8 bf16 values in a float4) or one element: added in fp32, rounded once
+template <typename T>
+__device__ __forceinline__ void add_rows(float4 &v, const float4 &old) {
+    typename Elt<T>::Acc acc = Elt<T>::widen(v);
+    Elt<T>::add(acc, old);
+    v = Elt<T>::pack(acc);
+}
+template <typename T>
+__device__ __forceinline__ void add_rows(T &v, const T &old) {
+    v = Elt<T>::from_f(Elt<T>::to_f(v) + Elt<T>::to_f(old));
+}
+
+// T: element type of the tiles; VT: what one lane moves at once (float4, or a single T when k is not a multiple of a vector)
+template <typename T, typename VT, int G, bool ACC, bool MULTI>
 __global__ void __launch_bounds__(256) k_gather_rows(VT *__restrict__ dst, const VT *__restrict__ src, MultiSrc ms,
                                                      const int *__restrict__ map, long long n_rows, int vec_per_row) {
     constexpr int RPW = 32 / G;
@@ -1314,14 +1402,7 @@ __global__ void __launch_bounds__(256) k_gather_rows(VT *__restrict__ dst, const
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
                 if (v0 + j * G < vec_per_row) {
-                    if (ACC) {
-                        VT old = dp[v0 + j * G];
-                        if constexpr (sizeof(VT) == 16) {
-                            f4_add(val[j], old);
-                        } else {
-                            val[j] += old;
-                        }
-                    }
+                    if (ACC) add_rows<T>(val[j], dp[v0 + j * G]);
                     dp[v0 + j * G] = val[j];
                 }
             }
@@ -1581,10 +1662,10 @@ struct TileLaunch {
     int rpg_req = 0;                 // 0 = default rows per lane group, 1 / 2 forced
 };
 
-template <int G, int VPL, int OUT, bool ACC, int TR, int TN, int RPG, int MINB, bool DUALX>
+template <typename T, int G, int VPL, int OUT, bool ACC, int TR, int TN, int RPG, int MINB, bool DUALX>
 int launch_tiles_one(arrow_ctx *ctx, const TileArgs &t) {
     constexpr size_t SMEM = TileCfg<TR, TN>::SMEM_BYTES;
-    auto fn = k_spmm_tiles<G, VPL, OUT, ACC, TR, TN, RPG, MINB, DUALX>;
+    auto fn = k_spmm_tiles<T, G, VPL, OUT, ACC, TR, TN, RPG, MINB, DUALX>;
     static bool attr_set[64] = {};            /* function attributes are per device */
     static int occ_dev[64] = {};
     const int dv = ctx->device & 63;
@@ -1611,10 +1692,10 @@ int launch_tiles_one(arrow_ctx *ctx, const TileArgs &t) {
     return ARROW_OK;
 }
 
-template <int G, int VPL, bool ROWMAP, bool ACC, int TR, int TN>
+template <typename T, int G, int VPL, bool ROWMAP, bool ACC, int TR, int TN>
 int launch_tiles_v1(arrow_ctx *ctx, const TileArgs &t) {
     constexpr size_t SMEM = TileCfg<TR, TN>::SMEM_BYTES;
-    auto fn = k_spmm_tiles_v1<G, VPL, ROWMAP, ACC, TR, TN>;
+    auto fn = k_spmm_tiles_v1<T, G, VPL, ROWMAP, ACC, TR, TN>;
     static bool attr_set[64] = {};
     static int occ_dev[64] = {};
     const int dv = ctx->device & 63;
@@ -1634,65 +1715,92 @@ int launch_tiles_v1(arrow_ctx *ctx, const TileArgs &t) {
     return ARROW_OK;
 }
 
-template <int G, int VPL, int TR, int TN, int RPG, int MINB>
+template <typename T, int G, int VPL, int TR, int TN, int RPG, int MINB>
 int launch_tiles_gv(arrow_ctx *ctx, const TileArgs &t, const TileLaunch &L) {
-    if (L.out_mode == OUT_ROWPTR) {
-        // the multi-GPU fused path: row-pointer epilogue, optionally the [recv region | local tile] dual X base
-        if (L.acc) return fail(ctx, ARROW_ERR_UNSUPPORTED, "row-pointer epilogue does not accumulate");
-        if (L.dualx) return launch_tiles_one<G, VPL, OUT_ROWPTR, false, TR, TN, RPG, MINB, true>(ctx, t);
-        return launch_tiles_one<G, VPL, OUT_ROWPTR, false, TR, TN, RPG, MINB, false>(ctx, t);
-    }
-    if (L.dualx) {
-        if (L.out_mode != OUT_IDENTITY || L.acc) return fail(ctx, ARROW_ERR_UNSUPPORTED, "dual X base needs a plain or row-pointer epilogue");
-        return launch_tiles_one<G, VPL, OUT_IDENTITY, false, TR, TN, RPG, MINB, true>(ctx, t);
-    }
-    if constexpr (RPG == 2) {
-        // the two-rows-per-group family exists for plain and row-pointer launches (the narrow-k fast path)
-        if (L.out_mode == OUT_IDENTITY && !L.acc) return launch_tiles_one<G, VPL, OUT_IDENTITY, false, TR, TN, 2, MINB, false>(ctx, t);
-        return launch_tiles_gv<G, VPL, TR, TN, 1, 4>(ctx, t, L);
-    } else {
-        const bool rowmap = L.out_mode == OUT_ROWMAP;
-        if (ctx->tile_kernel == 1) {
-            if (rowmap && L.acc) return launch_tiles_v1<G, VPL, true, true, TR, TN>(ctx, t);
-            if (rowmap) return launch_tiles_v1<G, VPL, true, false, TR, TN>(ctx, t);
-            if (L.acc) return launch_tiles_v1<G, VPL, false, true, TR, TN>(ctx, t);
-            return launch_tiles_v1<G, VPL, false, false, TR, TN>(ctx, t);
+    if constexpr (is_bf16<T>()) {
+        // bf16 launches are one-GPU launches (no row pointers, no dual X base; refused before this point) and always run
+        // the round-1 kernel, except the paired-row shape
+        if constexpr (RPG == 2) {
+            if (L.out_mode == OUT_IDENTITY && !L.acc) return launch_tiles_one<T, G, VPL, OUT_IDENTITY, false, TR, TN, 2, MINB, false>(ctx, t);
         }
-        if (rowmap && L.acc) return launch_tiles_one<G, VPL, OUT_ROWMAP, true, TR, TN, 1, MINB, false>(ctx, t);
-        if (rowmap) return launch_tiles_one<G, VPL, OUT_ROWMAP, false, TR, TN, 1, MINB, false>(ctx, t);
-        if (L.acc) return launch_tiles_one<G, VPL, OUT_IDENTITY, true, TR, TN, 1, MINB, false>(ctx, t);
-        return launch_tiles_one<G, VPL, OUT_IDENTITY, false, TR, TN, 1, MINB, false>(ctx, t);
+        const bool rowmap = L.out_mode == OUT_ROWMAP;
+        if (rowmap && L.acc) return launch_tiles_v1<T, G, VPL, true, true, TR, TN>(ctx, t);
+        if (rowmap) return launch_tiles_v1<T, G, VPL, true, false, TR, TN>(ctx, t);
+        if (L.acc) return launch_tiles_v1<T, G, VPL, false, true, TR, TN>(ctx, t);
+        return launch_tiles_v1<T, G, VPL, false, false, TR, TN>(ctx, t);
+    } else {
+        if (L.out_mode == OUT_ROWPTR) {
+            // the multi-GPU fused path: row-pointer epilogue, optionally the [recv region | local tile] dual X base
+            if (L.acc) return fail(ctx, ARROW_ERR_UNSUPPORTED, "row-pointer epilogue does not accumulate");
+            if (L.dualx) return launch_tiles_one<T, G, VPL, OUT_ROWPTR, false, TR, TN, RPG, MINB, true>(ctx, t);
+            return launch_tiles_one<T, G, VPL, OUT_ROWPTR, false, TR, TN, RPG, MINB, false>(ctx, t);
+        }
+        if (L.dualx) {
+            if (L.out_mode != OUT_IDENTITY || L.acc) return fail(ctx, ARROW_ERR_UNSUPPORTED, "dual X base needs a plain or row-pointer epilogue");
+            return launch_tiles_one<T, G, VPL, OUT_IDENTITY, false, TR, TN, RPG, MINB, true>(ctx, t);
+        }
+        if constexpr (RPG == 2) {
+            // the two-rows-per-group family exists for plain and row-pointer launches (the narrow-k fast path)
+            if (L.out_mode == OUT_IDENTITY && !L.acc) return launch_tiles_one<T, G, VPL, OUT_IDENTITY, false, TR, TN, 2, MINB, false>(ctx, t);
+            return launch_tiles_gv<T, G, VPL, TR, TN, 1, 4>(ctx, t, L);
+        } else {
+            const bool rowmap = L.out_mode == OUT_ROWMAP;
+            if (ctx->tile_kernel == 1) {
+                if (rowmap && L.acc) return launch_tiles_v1<T, G, VPL, true, true, TR, TN>(ctx, t);
+                if (rowmap) return launch_tiles_v1<T, G, VPL, true, false, TR, TN>(ctx, t);
+                if (L.acc) return launch_tiles_v1<T, G, VPL, false, true, TR, TN>(ctx, t);
+                return launch_tiles_v1<T, G, VPL, false, false, TR, TN>(ctx, t);
+            }
+            if (rowmap && L.acc) return launch_tiles_one<T, G, VPL, OUT_ROWMAP, true, TR, TN, 1, MINB, false>(ctx, t);
+            if (rowmap) return launch_tiles_one<T, G, VPL, OUT_ROWMAP, false, TR, TN, 1, MINB, false>(ctx, t);
+            if (L.acc) return launch_tiles_one<T, G, VPL, OUT_IDENTITY, true, TR, TN, 1, MINB, false>(ctx, t);
+            return launch_tiles_one<T, G, VPL, OUT_IDENTITY, false, TR, TN, 1, MINB, false>(ctx, t);
+        }
     }
 }
 
-// (lanes per row, float4 per lane) for a k4 = k/4; vpl_req = 0 picks the default
+// (lanes per row, 16-byte vectors per lane) for k4 vectors per row; vpl_req = 0 picks the default.  The shape follows the row's
+// bytes, so a bf16 row of k columns is served like an fp32 row of k/2 -- except that a bf16 vector needs 8 fp32 accumulators
+// where fp32 needs 4: VPL <= 2 keeps accumulators plus the gathers in flight (32 registers of X data per lane in every
+// shape) within the 64 registers of __launch_bounds__(256, 4).
+template <typename T>
 int launch_tiles(arrow_ctx *ctx, TileArgs &t, const Csr *A, const TileLaunch &L) {
     const int k4 = t.a.k4;
     int vpl = L.vpl_req;
     // measured on B200 (profiles/r01_kernel_sweep.md): ~8 lanes per row is the sweet spot
     if (vpl != 1 && vpl != 2 && vpl != 4) vpl = (k4 >= 32) ? 4 : (k4 >= 8 ? 2 : 1);
+    if (is_bf16<T>() && vpl > 2) vpl = 2;
     while (vpl > 1 && k4 < vpl) vpl >>= 1;
     int lanes = (k4 + vpl - 1) / vpl;                 // lanes needed per row
     if (lanes > 32) { vpl = (k4 + 31) / 32 <= 2 ? 2 : 4; lanes = (k4 + vpl - 1) / vpl; }
     int g = 1;
     while (g < lanes) g <<= 1;
-    const bool big = (k4 <= 8) && ctx->big_tiles && A->n_tiles_big > 0;     // k <= 32
+    const bool big = (k4 <= 8) && ctx->big_tiles && A->n_tiles_big > 0;     // rows of <= 128 bytes (fp32 k <= 32, bf16 k <= 64)
     if (big) { t.tiles = A->tiles_big; t.n_tiles = A->n_tiles_big; }
     // measured at 10M rows (profiles/r02_kernel_sweep.md): pairs win at k = 32 (+3.5 %), lose at k = 16 (-10 %)
     int rpg = L.rpg_req ? L.rpg_req : (ctx->rows_per_group ? ctx->rows_per_group : (vpl == 2 ? 2 : 1));
     if (!big || rpg != 2) rpg = 1;                                           // pairs need >= 2 passes per tile
 #define TL(GG, VV)                                                                                       \
-    if (g == GG && vpl == VV) return launch_tiles_gv<GG, VV, TILE_ROWS, TILE_NNZ, 1, 4>(ctx, t, L)
+    if (g == GG && vpl == VV) return launch_tiles_gv<T, GG, VV, TILE_ROWS, TILE_NNZ, 1, 4>(ctx, t, L)
 #define TLB(GG, VV)                                                                                      \
-    if (big && rpg == 1 && g == GG && vpl == VV) return launch_tiles_gv<GG, VV, TILE_ROWS_BIG, TILE_NNZ_BIG, 1, 4>(ctx, t, L)
+    if (big && rpg == 1 && g == GG && vpl == VV) return launch_tiles_gv<T, GG, VV, TILE_ROWS_BIG, TILE_NNZ_BIG, 1, 4>(ctx, t, L)
 #define TLP(GG, VV)                                                                                      \
-    if (big && rpg == 2 && g == GG && vpl == VV) return launch_tiles_gv<GG, VV, TILE_ROWS_BIG, TILE_NNZ_BIG, 2, 4>(ctx, t, L)
-    TLP(4, 1); TLP(8, 1); TLP(2, 2); TLP(4, 2);
-    if (rpg == 2) rpg = 1;                                                   // no paired kernel for this shape
-    TLB(1, 1); TLB(2, 1); TLB(4, 1); TLB(8, 1); TLB(1, 2); TLB(2, 2); TLB(4, 2); TLB(1, 4); TLB(2, 4);
-    TL(1, 1); TL(2, 1); TL(4, 1); TL(8, 1); TL(16, 1); TL(32, 1);
-    TL(1, 2); TL(2, 2); TL(4, 2); TL(8, 2); TL(16, 2); TL(32, 2);
-    TL(1, 4); TL(2, 4); TL(4, 4); TL(8, 4); TL(16, 4);
+    if (big && rpg == 2 && g == GG && vpl == VV) return launch_tiles_gv<T, GG, VV, TILE_ROWS_BIG, TILE_NNZ_BIG, 2, 4>(ctx, t, L)
+    if constexpr (is_bf16<T>()) {
+        // the shapes the defaults reach for k <= 256 (k = 16: 2 x 1, 32: 4 x 1, 64: 4 x 2 paired, 128: 8 x 2, 256: 16 x 2),
+        // plus those of big tiles off / one row per group; other forced shapes are refused below
+        TLP(4, 2);
+        if (rpg == 2) rpg = 1;
+        TLB(1, 1); TLB(2, 1); TLB(4, 1); TLB(8, 1); TLB(4, 2);
+        TL(1, 1); TL(2, 1); TL(4, 1); TL(8, 1); TL(4, 2); TL(8, 2); TL(16, 2);
+    } else {
+        TLP(4, 1); TLP(8, 1); TLP(2, 2); TLP(4, 2);
+        if (rpg == 2) rpg = 1;                                                   // no paired kernel for this shape
+        TLB(1, 1); TLB(2, 1); TLB(4, 1); TLB(8, 1); TLB(1, 2); TLB(2, 2); TLB(4, 2); TLB(1, 4); TLB(2, 4);
+        TL(1, 1); TL(2, 1); TL(4, 1); TL(8, 1); TL(16, 1); TL(32, 1);
+        TL(1, 2); TL(2, 2); TL(4, 2); TL(8, 2); TL(16, 2); TL(32, 2);
+        TL(1, 4); TL(2, 4); TL(4, 4); TL(8, 4); TL(16, 4);
+    }
 #undef TL
 #undef TLB
 #undef TLP
@@ -2195,12 +2303,18 @@ int arrow_map_d2h(arrow_ctx *ctx, int map, int32_t *host, int64_t n) {
 
 // ---- dense --------------------------------------------------------------------------------------
 int arrow_dense_alloc(arrow_ctx *ctx, int64_t rows, int k, int *buf_out) {
+    return arrow_dense_alloc_dtype(ctx, rows, k, ARROW_DTYPE_F32, buf_out);
+}
+
+int arrow_dense_alloc_dtype(arrow_ctx *ctx, int64_t rows, int k, int dtype, int *buf_out) {
     CHECK_CTX(ctx);
     if (!buf_out || rows < 0 || k < 1) return fail(ctx, ARROW_ERR_ARG, "bad dense shape %lld x %d", (long long)rows, k);
+    if (dtype != ARROW_DTYPE_F32 && dtype != ARROW_DTYPE_BF16) return fail(ctx, ARROW_ERR_ARG, "unknown dtype %d", dtype);
     DenseBuf d;
     d.rows = rows;
     d.k = k;
-    const size_t bytes = std::max<size_t>((size_t)rows * (size_t)k * 4, 16);
+    d.dtype = dtype;
+    const size_t bytes = std::max<size_t>((size_t)rows * (size_t)k * d.esize(), 16);
     cudaError_t e = cudaMalloc(&d.p, bytes);
     if (e != cudaSuccess) {
         cudaGetLastError();
@@ -2213,6 +2327,15 @@ int arrow_dense_alloc(arrow_ctx *ctx, int64_t rows, int k, int *buf_out) {
     const int h = new_slot(ctx->dense);
     ctx->dense[h] = d;
     *buf_out = h;
+    return ARROW_OK;
+}
+
+int arrow_dense_dtype(arrow_ctx *ctx, int buf, int *dtype) {
+    CHECK_CTX(ctx);
+    DenseBuf *d = get_dense(ctx, buf);
+    if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
+    if (!dtype) return fail(ctx, ARROW_ERR_ARG, "dtype is null");
+    *dtype = d->dtype;
     return ARROW_OK;
 }
 
@@ -2234,7 +2357,11 @@ int arrow_dense_fill(arrow_ctx *ctx, int buf, float value) {
     const long long n = (long long)d->rows * d->k;
     if (n == 0) return ARROW_OK;
     if (value == 0.f) {
-        CUDA_TRY(ctx, cudaMemsetAsync(d->p, 0, (size_t)n * 4, ctx->stream));
+        CUDA_TRY(ctx, cudaMemsetAsync(d->p, 0, (size_t)n * d->esize(), ctx->stream));
+    } else if (d->dtype == ARROW_DTYPE_BF16) {
+        k_fill<bf16><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(reinterpret_cast<bf16 *>(d->p), __float2bfloat16_rn(value), n);
+        ctx->launches++;
+        CUDA_TRY(ctx, cudaGetLastError());
     } else {
         k_fill<float><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(d->p, value, n);
         ctx->launches++;
@@ -2249,6 +2376,7 @@ int arrow_dense_h2d(arrow_ctx *ctx, int buf, int64_t row0, int64_t rows, const f
     if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
     if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows)
         return fail(ctx, ARROW_ERR_ARG, "h2d rows [%lld,%lld) outside tile of %lld rows", (long long)row0, (long long)(row0 + rows), (long long)d->rows);
+    REQUIRE_F32(ctx, d, "arrow_dense_h2d (float rows; arrow_dense_put copies any dtype)");
     if (rows == 0) return ARROW_OK;
     CUDA_TRY(ctx, cudaMemcpyAsync(d->p + (size_t)row0 * d->k, host, (size_t)rows * d->k * 4, cudaMemcpyHostToDevice, ctx->stream));
     return ARROW_OK;
@@ -2260,6 +2388,7 @@ int arrow_dense_d2h(arrow_ctx *ctx, int buf, int64_t row0, int64_t rows, float *
     if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
     if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows)
         return fail(ctx, ARROW_ERR_ARG, "d2h rows [%lld,%lld) outside tile of %lld rows", (long long)row0, (long long)(row0 + rows), (long long)d->rows);
+    REQUIRE_F32(ctx, d, "arrow_dense_d2h (float rows; arrow_dense_get copies any dtype)");
     if (rows == 0) return ARROW_OK;
     CUDA_TRY(ctx, cudaMemcpyAsync(host, d->p + (size_t)row0 * d->k, (size_t)rows * d->k * 4, cudaMemcpyDeviceToHost, ctx->stream));
     return ARROW_OK;
@@ -2270,10 +2399,11 @@ int arrow_dense_copy(arrow_ctx *ctx, int dst, int64_t dst_row0, int src, int64_t
     DenseBuf *a = get_dense(ctx, dst), *b = get_dense(ctx, src);
     if (!a || !b) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle");
     if (a->k != b->k) return fail(ctx, ARROW_ERR_ARG, "feature width mismatch %d vs %d", a->k, b->k);
+    if (a->dtype != b->dtype) return fail(ctx, ARROW_ERR_ARG, "copy between tiles of different dtype (%d vs %d)", b->dtype, a->dtype);
     if (rows < 0 || dst_row0 < 0 || src_row0 < 0 || dst_row0 + rows > a->rows || src_row0 + rows > b->rows)
         return fail(ctx, ARROW_ERR_ARG, "copy range outside tiles");
     if (rows == 0) return ARROW_OK;
-    CUDA_TRY(ctx, cudaMemcpyAsync(a->p + (size_t)dst_row0 * a->k, b->p + (size_t)src_row0 * b->k, (size_t)rows * a->k * 4,
+    CUDA_TRY(ctx, cudaMemcpyAsync(a->row(dst_row0), b->row(src_row0), (size_t)rows * a->k * a->esize(),
                                   cudaMemcpyDeviceToDevice, cur_stream(ctx)));
     return ARROW_OK;
 }
@@ -2358,6 +2488,11 @@ int arrow_spmm_add(arrow_ctx *ctx, int csr, int x_buf, int c_buf, int add_buf, i
 
 int arrow_spmm_ex(arrow_ctx *ctx, int csr, int x_buf, int x2_buf, int64_t x_split, int c_buf, int out_table,
                   int add_buf, int add_map, int variant) {
+    CHECK_CTX(ctx);
+    for (int h : {x_buf, x2_buf, c_buf, add_buf}) {
+        const DenseBuf *d = get_dense(ctx, h);
+        if (d && d->dtype != ARROW_DTYPE_F32) return fail(ctx, ARROW_ERR_ARG, "arrow_spmm_ex (N-GPU path) needs fp32 tiles; buffer %d is bf16", h);
+    }
     SpmmCall q;
     q.csr = csr; q.x_buf = x_buf; q.x2_buf = x2_buf; q.x_split = x_split; q.c_buf = c_buf; q.out_table = out_table;
     q.add_buf = add_buf; q.add_map = add_map; q.variant = variant;
@@ -2383,9 +2518,11 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
     } else if (!C) {
         return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle (c=%d)", q.c_buf);
     }
+    const bool bf = X->dtype == ARROW_DTYPE_BF16;
     if (C) {
         if (X->k != C->k) return fail(ctx, ARROW_ERR_ARG, "X has %d feature columns, C has %d", X->k, C->k);
         if (X->p == C->p) return fail(ctx, ARROW_ERR_ARG, "X and C must not alias");
+        if (X->dtype != C->dtype) return fail(ctx, ARROW_ERR_ARG, "X and C differ in dtype (%d vs %d)", X->dtype, C->dtype);
     }
     DenseBuf *X2 = nullptr;
     if (q.x2_buf >= 0) {
@@ -2423,7 +2560,7 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
     a.rowmap = rm ? rm->p : nullptr;
     a.n_rows = A->n_rows;
     a.k = k;
-    a.k4 = k / 4;
+    a.k4 = k / (bf ? Elt<bf16>::PER_VEC : Elt<float>::PER_VEC);
     a.long_threshold = A->long_threshold;
     a.add_src = nullptr;
     a.add_map = nullptr;
@@ -2435,6 +2572,7 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
         IdxMap *am = get_map(ctx, q.add_map);
         if (!S || !am) return fail(ctx, ARROW_ERR_HANDLE, "bad addend handles (buf=%d map=%d)", q.add_buf, q.add_map);
         if (S->k != k) return fail(ctx, ARROW_ERR_ARG, "addend has %d feature columns, expected %d", S->k, k);
+        if (S->dtype != X->dtype) return fail(ctx, ARROW_ERR_ARG, "addend and X differ in dtype (%d vs %d)", S->dtype, X->dtype);
         if (am->n < A->n_rows) return fail(ctx, ARROW_ERR_ARG, "addend map has %lld entries, block has %lld rows", (long long)am->n, (long long)A->n_rows);
         if (am->limit > S->rows) return fail(ctx, ARROW_ERR_ARG, "addend map reaches row %lld, addend tile has %lld rows", (long long)am->limit, (long long)S->rows);
         if (C && S->p == C->p) return fail(ctx, ARROW_ERR_ARG, "addend and C must not alias");
@@ -2449,9 +2587,10 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
     // the epilogue gather-add, the dual X base and the row-pointer epilogue live in the tile / generic / long kernels
     if ((a.add_map != nullptr || X2 || OT) && variant != 3) variant = 3;
     if (variant < 0 || variant > 3) return fail(ctx, ARROW_ERR_ARG, "unknown variant %d", variant);
+    if (bf && variant != ARROW_VARIANT_TILES) return fail(ctx, ARROW_ERR_UNSUPPORTED, "bf16 tiles run the tile kernel only (variant %d)", variant);
     const bool fused_launch = rm != nullptr || acc || OT != nullptr || X2 != nullptr || a.add_map != nullptr;
 
-    const bool vec_ok = (k % 4 == 0) && k <= 256;
+    const bool vec_ok = (k % (bf ? 8 : 4) == 0) && k <= 256;
     if (!vec_ok) {
         const long long ctas = (A->n_rows + 7) / 8;
 #define LAUNCH_G(KERNEL)                                                                              \
@@ -2460,10 +2599,17 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
         int grid = grid_for(ctx, (const void *)fn, 256, 0, ctas);                                     \
         fn<<<grid, 256, 0, stream>>>(a);                                                              \
     } while (0)
-        if (rm && acc) LAUNCH_G((k_spmm_generic<true, true>));
-        else if (rm) LAUNCH_G((k_spmm_generic<true, false>));
-        else if (acc) LAUNCH_G((k_spmm_generic<false, true>));
-        else LAUNCH_G((k_spmm_generic<false, false>));
+        if (bf) {
+            if (rm && acc) LAUNCH_G((k_spmm_generic<bf16, true, true>));
+            else if (rm) LAUNCH_G((k_spmm_generic<bf16, true, false>));
+            else if (acc) LAUNCH_G((k_spmm_generic<bf16, false, true>));
+            else LAUNCH_G((k_spmm_generic<bf16, false, false>));
+        } else {
+            if (rm && acc) LAUNCH_G((k_spmm_generic<float, true, true>));
+            else if (rm) LAUNCH_G((k_spmm_generic<float, true, false>));
+            else if (acc) LAUNCH_G((k_spmm_generic<float, false, true>));
+            else LAUNCH_G((k_spmm_generic<float, false, false>));
+        }
 #undef LAUNCH_G
         ctx->launches++;
     } else if (variant == 3) {
@@ -2482,7 +2628,7 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
             L.dualx = X2 != nullptr;
             L.vpl_req = vpl_req;
             L.rpg_req = rpg_req;
-            int rc = launch_tiles(ctx, t, A, L);
+            int rc = bf ? launch_tiles<bf16>(ctx, t, A, L) : launch_tiles<float>(ctx, t, A, L);
             if (rc != ARROW_OK) return rc;
         }
     } else if (variant == ARROW_VARIANT_TMA && k >= 32 && k <= 128) {
@@ -2522,17 +2668,30 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
         la.X2 = a.X2;
         la.x_split = a.x_split;
         const size_t smem = (size_t)8 * k * 4;
+        auto partial = bf ? k_spmm_long_partial<bf16> : k_spmm_long_partial<float>;
         if (smem > 48 * 1024)
-            CUDA_TRY(ctx, cudaFuncSetAttribute(k_spmm_long_partial, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_spmm_long_partial<<<A->n_long_tasks, 256, smem, stream>>>(la);
+            CUDA_TRY(ctx, cudaFuncSetAttribute(partial, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        partial<<<A->n_long_tasks, 256, smem, stream>>>(la);
         ctx->launches++;
         const int *rmp = rm ? rm->p : nullptr;
         float *cp = C ? C->p : nullptr;
         float *scr = ctx->long_scratch[lane];
-        if (rm && acc) k_spmm_long_reduce<true, true><<<A->n_long_rows, 128, 0, stream>>>(A->long_rows, A->long_first, scr, cp, rmp, k, a.add_src, a.add_map, a.out_ptr);
-        else if (rm) k_spmm_long_reduce<true, false><<<A->n_long_rows, 128, 0, stream>>>(A->long_rows, A->long_first, scr, cp, rmp, k, a.add_src, a.add_map, a.out_ptr);
-        else if (acc) k_spmm_long_reduce<false, true><<<A->n_long_rows, 128, 0, stream>>>(A->long_rows, A->long_first, scr, cp, rmp, k, a.add_src, a.add_map, a.out_ptr);
-        else k_spmm_long_reduce<false, false><<<A->n_long_rows, 128, 0, stream>>>(A->long_rows, A->long_first, scr, cp, rmp, k, a.add_src, a.add_map, a.out_ptr);
+#define LAUNCH_R(TT, RM, AC)                                                                                        \
+    k_spmm_long_reduce<TT, RM, AC><<<A->n_long_rows, 128, 0, stream>>>(A->long_rows, A->long_first, scr,            \
+                                                                      reinterpret_cast<TT *>(cp), rmp, k,           \
+                                                                      reinterpret_cast<const TT *>(a.add_src), a.add_map, a.out_ptr)
+        if (bf) {
+            if (rm && acc) LAUNCH_R(bf16, true, true);
+            else if (rm) LAUNCH_R(bf16, true, false);
+            else if (acc) LAUNCH_R(bf16, false, true);
+            else LAUNCH_R(bf16, false, false);
+        } else {
+            if (rm && acc) LAUNCH_R(float, true, true);
+            else if (rm) LAUNCH_R(float, true, false);
+            else if (acc) LAUNCH_R(float, false, true);
+            else LAUNCH_R(float, false, false);
+        }
+#undef LAUNCH_R
         ctx->launches++;
         CUDA_TRY(ctx, cudaGetLastError());
     }
@@ -2551,6 +2710,7 @@ int arrow_ptrtable_upload(arrow_ctx *ctx, const int *bufs, int n_bufs, const int
     for (int b = 0; b < n_bufs; ++b) {
         DenseBuf *d = get_dense(ctx, bufs[b]);
         if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", bufs[b]);
+        REQUIRE_F32(ctx, d, "arrow_ptrtable_upload (N-GPU path)");
         if (b == 0) k = d->k;
         else if (d->k != k) return fail(ctx, ARROW_ERR_ARG, "tiles of a pointer table must share the feature width");
         bases[b] = (unsigned long long)d->p;
@@ -2613,8 +2773,10 @@ static int gather_common(arrow_ctx *ctx, DenseBuf *D, const float *src, const Mu
     const long long n_rows = m->n;
     if (n_rows == 0) return ARROW_OK;
     const int k = D->k;
-    const bool vec = (k % 4 == 0);
-    const int vpr = vec ? k / 4 : k;
+    const bool bf = D->dtype == ARROW_DTYPE_BF16;
+    const int per_vec = bf ? Elt<bf16>::PER_VEC : Elt<float>::PER_VEC;
+    const bool vec = (k % per_vec == 0);
+    const int vpr = vec ? k / per_vec : k;
     int g = 1;
     while (g < vpr && g < 32) g <<= 1;                       // lanes per row
     if (g > 8 && vpr <= 32) g = 8;                           // 8 lanes x 4 vectors cover k <= 128 in one pass
@@ -2622,26 +2784,29 @@ static int gather_common(arrow_ctx *ctx, DenseBuf *D, const float *src, const Mu
     const long long rows_per_cta = (threads / 32) * (32 / g);
     int grid = (int)std::min<long long>((n_rows + rows_per_cta - 1) / rows_per_cta, (long long)ctx->sm_count * 8);
     grid = std::max(grid, 1);
-#define LAUNCH_GA(VT, GG, ACCV, MULTIV)                                                                          \
-    k_gather_rows<VT, GG, ACCV, MULTIV><<<grid, threads, 0, cur_stream(ctx)>>>(reinterpret_cast<VT *>(D->p),     \
+#define LAUNCH_GA(T, VT, GG, ACCV, MULTIV)                                                                       \
+    k_gather_rows<T, VT, GG, ACCV, MULTIV><<<grid, threads, 0, cur_stream(ctx)>>>(reinterpret_cast<VT *>(D->p),  \
                                                                            reinterpret_cast<const VT *>(src), ms, m->p, n_rows, vpr)
-#define DISPATCH_G(VT, ACCV, MULTIV)                                                                             \
+#define DISPATCH_G(T, VT, ACCV, MULTIV)                                                                          \
     do {                                                                                                         \
         switch (g) {                                                                                             \
-            case 1: LAUNCH_GA(VT, 1, ACCV, MULTIV); break;                                                       \
-            case 2: LAUNCH_GA(VT, 2, ACCV, MULTIV); break;                                                       \
-            case 4: LAUNCH_GA(VT, 4, ACCV, MULTIV); break;                                                       \
-            case 8: LAUNCH_GA(VT, 8, ACCV, MULTIV); break;                                                       \
-            case 16: LAUNCH_GA(VT, 16, ACCV, MULTIV); break;                                                     \
-            default: LAUNCH_GA(VT, 32, ACCV, MULTIV); break;                                                     \
+            case 1: LAUNCH_GA(T, VT, 1, ACCV, MULTIV); break;                                                    \
+            case 2: LAUNCH_GA(T, VT, 2, ACCV, MULTIV); break;                                                    \
+            case 4: LAUNCH_GA(T, VT, 4, ACCV, MULTIV); break;                                                    \
+            case 8: LAUNCH_GA(T, VT, 8, ACCV, MULTIV); break;                                                    \
+            case 16: LAUNCH_GA(T, VT, 16, ACCV, MULTIV); break;                                                  \
+            default: LAUNCH_GA(T, VT, 32, ACCV, MULTIV); break;                                                  \
         }                                                                                                        \
     } while (0)
-    if (vec) {
-        if (multi) { if (acc) DISPATCH_G(float4, true, true); else DISPATCH_G(float4, false, true); }
-        else       { if (acc) DISPATCH_G(float4, true, false); else DISPATCH_G(float4, false, false); }
+    if (bf) {                           // one-GPU exchanges only (arrow_gather_rows_multi refuses bf16)
+        if (vec) { if (acc) DISPATCH_G(bf16, float4, true, false); else DISPATCH_G(bf16, float4, false, false); }
+        else     { if (acc) DISPATCH_G(bf16, bf16, true, false); else DISPATCH_G(bf16, bf16, false, false); }
+    } else if (vec) {
+        if (multi) { if (acc) DISPATCH_G(float, float4, true, true); else DISPATCH_G(float, float4, false, true); }
+        else       { if (acc) DISPATCH_G(float, float4, true, false); else DISPATCH_G(float, float4, false, false); }
     } else {
-        if (multi) { if (acc) DISPATCH_G(float, true, true); else DISPATCH_G(float, false, true); }
-        else       { if (acc) DISPATCH_G(float, true, false); else DISPATCH_G(float, false, false); }
+        if (multi) { if (acc) DISPATCH_G(float, float, true, true); else DISPATCH_G(float, float, false, true); }
+        else       { if (acc) DISPATCH_G(float, float, true, false); else DISPATCH_G(float, float, false, false); }
     }
 #undef DISPATCH_G
 #undef LAUNCH_GA
@@ -2657,6 +2822,7 @@ int arrow_gather_rows(arrow_ctx *ctx, int dst_buf, int src_buf, int map, int fla
     if (!D || !S) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle (dst=%d src=%d)", dst_buf, src_buf);
     if (!m) return fail(ctx, ARROW_ERR_HANDLE, "bad map handle %d", map);
     if (D->k != S->k) return fail(ctx, ARROW_ERR_ARG, "feature width mismatch %d vs %d", D->k, S->k);
+    if (D->dtype != S->dtype) return fail(ctx, ARROW_ERR_ARG, "gather source and destination differ in dtype (%d vs %d)", S->dtype, D->dtype);
     if (D->p == S->p) return fail(ctx, ARROW_ERR_ARG, "gather source and destination must not alias");
     if (m->n > D->rows) return fail(ctx, ARROW_ERR_ARG, "map has %lld entries, destination has %lld rows", (long long)m->n, (long long)D->rows);
     if (m->limit > S->rows) return fail(ctx, ARROW_ERR_ARG, "map reaches row %lld, source has %lld rows", (long long)m->limit, (long long)S->rows);
@@ -2672,6 +2838,7 @@ int arrow_gather_rows_multi(arrow_ctx *ctx, int dst_buf, const int *src_bufs, co
     if (!D) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", dst_buf);
     if (!m) return fail(ctx, ARROW_ERR_HANDLE, "bad map handle %d", map);
     if (!src_bufs || !row_bounds || n_src < 1 || n_src > MAX_SRC) return fail(ctx, ARROW_ERR_ARG, "need 1..%d sources", MAX_SRC);
+    REQUIRE_F32(ctx, D, "arrow_gather_rows_multi (N-GPU path)");
     if (m->n > D->rows) return fail(ctx, ARROW_ERR_ARG, "map has %lld entries, destination has %lld rows", (long long)m->n, (long long)D->rows);
     MultiSrc ms;
     memset(&ms, 0, sizeof ms);
@@ -2680,6 +2847,7 @@ int arrow_gather_rows_multi(arrow_ctx *ctx, int dst_buf, const int *src_bufs, co
         DenseBuf *S = get_dense(ctx, src_bufs[s]);
         if (!S) return fail(ctx, ARROW_ERR_HANDLE, "bad source handle %d", src_bufs[s]);
         if (S->k != D->k) return fail(ctx, ARROW_ERR_ARG, "feature width mismatch in source %d", s);
+        REQUIRE_F32(ctx, S, "arrow_gather_rows_multi (N-GPU path)");
         if (row_bounds[s + 1] < row_bounds[s] || row_bounds[s + 1] - row_bounds[s] > S->rows)
             return fail(ctx, ARROW_ERR_ARG, "source %d owns %lld rows but its tile has %lld", s, (long long)(row_bounds[s + 1] - row_bounds[s]), (long long)S->rows);
         if (S->p == D->p) return fail(ctx, ARROW_ERR_ARG, "gather source and destination must not alias");
@@ -2699,6 +2867,7 @@ int arrow_push_rows(arrow_ctx *ctx, const int *dst_bufs, const int64_t *item_bou
     if (!S) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", src_buf);
     if (!m) return fail(ctx, ARROW_ERR_HANDLE, "bad map handle %d", map);
     if (!dst_bufs || !item_bounds || n_dst < 1 || n_dst > MAX_SRC) return fail(ctx, ARROW_ERR_ARG, "need 1..%d destinations", MAX_SRC);
+    REQUIRE_F32(ctx, S, "arrow_push_rows (N-GPU path)");
     if (m->limit > S->rows) return fail(ctx, ARROW_ERR_ARG, "map reaches row %lld, source has %lld rows", (long long)m->limit, (long long)S->rows);
     if (item_bounds[0] != 0 || item_bounds[n_dst] != m->n) return fail(ctx, ARROW_ERR_ARG, "item bounds must span [0, %lld]", (long long)m->n);
     MultiDst md;
@@ -2712,6 +2881,7 @@ int arrow_push_rows(arrow_ctx *ctx, const int *dst_bufs, const int64_t *item_bou
         DenseBuf *D = get_dense(ctx, dst_bufs[d]);
         if (!D) return fail(ctx, ARROW_ERR_HANDLE, "bad destination handle %d", dst_bufs[d]);
         if (D->k != S->k) return fail(ctx, ARROW_ERR_ARG, "feature width mismatch in destination %d", d);
+        REQUIRE_F32(ctx, D, "arrow_push_rows (N-GPU path)");
         if (cnt > D->rows) return fail(ctx, ARROW_ERR_ARG, "destination %d receives %lld rows but its region has %lld", d, (long long)cnt, (long long)D->rows);
         if (D->p == S->p) return fail(ctx, ARROW_ERR_ARG, "push source and destination must not alias");
         md.p[d] = D->p;
@@ -2758,6 +2928,7 @@ int arrow_reduce_rows(arrow_ctx *ctx, int dst_buf, int out_table, const int *src
     if (!src_bufs || n_src < 1 || n_src > MAX_SRC || rows < 0) return fail(ctx, ARROW_ERR_ARG, "need 1..%d sources", MAX_SRC);
     DenseBuf *D = dst_buf >= 0 ? get_dense(ctx, dst_buf) : nullptr;
     if (dst_buf >= 0 && !D) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", dst_buf);
+    if (D) REQUIRE_F32(ctx, D, "arrow_reduce_rows (N-GPU path)");
     PtrTable *OT = nullptr;
     if (out_table >= 0) {
         if (out_table >= (int)ctx->ptrtabs.size() || !ctx->ptrtabs[out_table].live)
@@ -2775,6 +2946,7 @@ int arrow_reduce_rows(arrow_ctx *ctx, int dst_buf, int out_table, const int *src
         DenseBuf *S = get_dense(ctx, src_bufs[s2]);
         if (!S) return fail(ctx, ARROW_ERR_HANDLE, "bad source handle %d", src_bufs[s2]);
         if (s2 == 0) k = S->k;
+        REQUIRE_F32(ctx, S, "arrow_reduce_rows (N-GPU path)");
         if (S->k != k || (D && D->k != k) || (OT && OT->k != k)) return fail(ctx, ARROW_ERR_ARG, "feature width mismatch in source %d", s2);
         if (S->rows < rows) return fail(ctx, ARROW_ERR_ARG, "source %d has %lld rows, %lld are reduced", s2, (long long)S->rows, (long long)rows);
         ms.p[s2] = S->p;
@@ -2817,6 +2989,7 @@ int arrow_ipc_export(arrow_ctx *ctx, int buf, void *handle) {
     DenseBuf *d = get_dense(ctx, buf);
     if (!d || !d->owned) return fail(ctx, ARROW_ERR_HANDLE, "ipc export needs a tile this context allocated (handle %d)", buf);
     if (!handle) return fail(ctx, ARROW_ERR_ARG, "handle is null");
+    REQUIRE_F32(ctx, d, "arrow_ipc_export (N-GPU path)");
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "ipc handle size");
     cudaIpcMemHandle_t h;
     CUDA_TRY(ctx, cudaIpcGetMemHandle(&h, d->p));
@@ -2892,6 +3065,7 @@ int arrow_dense_h2d_lane(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_
     DenseBuf *d = get_dense(ctx, buf);
     if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
     if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows) return fail(ctx, ARROW_ERR_ARG, "h2d range outside tile");
+    REQUIRE_F32(ctx, d, "arrow_dense_h2d_lane (float rows; arrow_dense_put copies any dtype)");
     cudaStream_t st;
     int rc = lane_stream(ctx, lane, &st);
     if (rc != ARROW_OK) return rc;
@@ -2904,10 +3078,37 @@ int arrow_dense_d2h_lane(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_
     DenseBuf *d = get_dense(ctx, buf);
     if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
     if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows) return fail(ctx, ARROW_ERR_ARG, "d2h range outside tile");
+    REQUIRE_F32(ctx, d, "arrow_dense_d2h_lane (float rows; arrow_dense_get copies any dtype)");
     cudaStream_t st;
     int rc = lane_stream(ctx, lane, &st);
     if (rc != ARROW_OK) return rc;
     if (rows) CUDA_TRY(ctx, cudaMemcpyAsync(host, d->p + (size_t)row0 * d->k, (size_t)rows * d->k * 4, cudaMemcpyDeviceToHost, st));
+    return ARROW_OK;
+}
+
+int arrow_dense_put(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_t rows, const void *host) {
+    CHECK_CTX(ctx);
+    DenseBuf *d = get_dense(ctx, buf);
+    if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
+    if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows)
+        return fail(ctx, ARROW_ERR_ARG, "put rows [%lld,%lld) outside tile of %lld rows", (long long)row0, (long long)(row0 + rows), (long long)d->rows);
+    cudaStream_t st;
+    int rc = lane_stream(ctx, lane, &st);
+    if (rc != ARROW_OK) return rc;
+    if (rows) CUDA_TRY(ctx, cudaMemcpyAsync(d->row(row0), host, (size_t)rows * d->k * d->esize(), cudaMemcpyHostToDevice, st));
+    return ARROW_OK;
+}
+
+int arrow_dense_get(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_t rows, void *host) {
+    CHECK_CTX(ctx);
+    DenseBuf *d = get_dense(ctx, buf);
+    if (!d) return fail(ctx, ARROW_ERR_HANDLE, "bad dense handle %d", buf);
+    if (!host || row0 < 0 || rows < 0 || row0 + rows > d->rows)
+        return fail(ctx, ARROW_ERR_ARG, "get rows [%lld,%lld) outside tile of %lld rows", (long long)row0, (long long)(row0 + rows), (long long)d->rows);
+    cudaStream_t st;
+    int rc = lane_stream(ctx, lane, &st);
+    if (rc != ARROW_OK) return rc;
+    if (rows) CUDA_TRY(ctx, cudaMemcpyAsync(host, d->row(row0), (size_t)rows * d->k * d->esize(), cudaMemcpyDeviceToHost, st));
     return ARROW_OK;
 }
 

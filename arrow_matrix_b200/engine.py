@@ -17,6 +17,10 @@ Two execution modes, same results:
   (``C_0[map_j[r]] += ...``); no gather kernel runs and levels > 0 never materialise their tiles.
   Chosen automatically when no non-zero of a level reads a row behind the sentinel (then both
   modes are mathematically identical); otherwise the engine stays in ``exchange`` mode.
+
+Feature and result tiles are float32 (default) or bfloat16 (``dtype``, ``set_dtype``); CSR values and all arithmetic stay
+float32, and every stored bf16 row is rounded once to nearest even (DESIGN.md, numerics of bf16 tiles).  bf16 host
+rows are CPU ``torch.bfloat16`` tensors.
 """
 from __future__ import annotations
 
@@ -47,11 +51,12 @@ class ArrowEngine:
     def __init__(self, decomposition: Sequence[Tuple[decomp.Level, np.ndarray]], width: int, k: int,
                  block_diagonal: bool = True, device: int = 0, mode: str = "auto", stream: Optional[int] = None,
                  variant: int = _lib.VARIANT_AUTO, n_blocks: Optional[Sequence[int]] = None,
-                 ctx: Optional[_lib.Context] = None, fused_style: str = "gather"):
+                 ctx: Optional[_lib.Context] = None, fused_style: str = "gather", dtype="float32"):
         if mode not in ("auto", "fused", "exchange"):
             raise ValueError(f"mode must be auto|fused|exchange, got {mode!r}")
         self.ctx = ctx if ctx is not None else _lib.Context(device, stream)
         self.width, self.k, self.variant = int(width), int(k), variant
+        self.dtype = _lib.dtype_name(dtype)
         if fused_style not in ("gather", "scatter"):
             raise ValueError("fused_style must be 'gather' or 'scatter'")
         self.fused_style = fused_style
@@ -106,12 +111,20 @@ class ArrowEngine:
     def _alloc_buffers(self):
         for j, st in enumerate(self.levels):
             if j == 0 or self.mode == "exchange":
-                st.bufs = [self.ctx.dense_alloc(st.rows, self.k), self.ctx.dense_alloc(st.rows, self.k)]
+                st.bufs = [self._tile(st.rows), self._tile(st.rows)]
                 st.xi, st.ci = 0, 0             # zero_rhs: X and C both zero (arrow_slim_mpi.py:354-394)
             if j > 0 and self.mode == "fused":
                 st.csr_fused = st.csr.remap_columns(st.cmap_dev, self.levels[0].rows)
                 if self.fused_style == "gather":
-                    st.cbuf = self.ctx.dense_alloc(st.rows, self.k)     # this level's result tile, written once per step
+                    st.cbuf = self._tile(st.rows)     # this level's result tile, written once per step
+
+    def _tile(self, rows: int) -> _lib.Dense:
+        return self.ctx.dense_alloc(rows, self.k, self.dtype)
+
+    @property
+    def itemsize(self) -> int:
+        """bytes per feature element"""
+        return 2 if self.dtype == "bfloat16" else 4
 
     def set_mode(self, mode: str):
         """Switch between 'fused' and 'exchange' (re-allocates level tiles; features are reset)."""
@@ -119,6 +132,21 @@ class ArrowEngine:
             return
         if mode == "fused" and not self.fused_ok:
             raise ValueError("fused mode is not valid for this decomposition")
+        self._release_buffers()
+        self.mode = mode
+        self._alloc_buffers()
+
+    def set_dtype(self, dtype):
+        """Switch the feature / result tiles between float32 and bfloat16 (re-allocates level tiles and streaming slots
+        like ``set_mode``; features are reset to zero)."""
+        dtype = _lib.dtype_name(dtype)
+        if dtype == self.dtype:
+            return
+        self._release_buffers()
+        self.dtype = dtype
+        self._alloc_buffers()
+
+    def _release_buffers(self):
         if hasattr(self, "_slots"):                 # streaming slots hold level-0 tiles of the old mode
             self.stream_drain()
             for b in self._slots[1]:
@@ -136,16 +164,15 @@ class ArrowEngine:
             if st.cbuf is not None:
                 st.cbuf.free()
                 st.cbuf = None
-        self.mode = mode
-        self._alloc_buffers()
 
     @property
     def n_rows(self) -> int:
         return self.levels[0].rows
 
     # -- features / results (level-0 row order, like the reference's per-rank tiles) -----------------
-    def set_features(self, X: np.ndarray, sync: bool = True):
-        """Level-0 feature tiles, concatenated (``B.set_features`` on every level-0 rank)."""
+    def set_features(self, X, sync: bool = True):
+        """Level-0 feature tiles, concatenated (``B.set_features`` on every level-0 rank).  A bf16 engine takes a CPU
+        bf16 tensor, or float32 rows it rounds to nearest even."""
         st = self.levels[0]
         if X.shape != (st.rows, self.k):
             raise ValueError(f"expected features of shape {(st.rows, self.k)}, got {X.shape}")
@@ -289,7 +316,7 @@ class ArrowEngine:
         """Enqueue one full iteration on host data: upload ``X_host`` -> ``step()`` -> download level-0 result
         into ``out_host``.  Returns immediately; uploads, compute and downloads of consecutive calls overlap
         (side copy streams ordered with events, two device slots).  Both arrays must be pinned
-        (``_lib.PinnedArray``) and must stay untouched until ``stream_drain()``; use at least two
+        (``_lib.PinnedArray``; for a bf16 engine the ``tensor`` of a ``_lib.PinnedTensor``) and must stay untouched until ``stream_drain()``; use at least two
         (X, out) pairs in rotation.  Results are identical to ``set_features(X); step(); result()``."""
         st = self.levels[0]
         if X_host.shape != (st.rows, self.k) or out_host.shape != (st.rows, self.k):
@@ -297,7 +324,7 @@ class ArrowEngine:
         ctx = self.ctx
         if not hasattr(self, "_slots"):
             # slot 0 re-uses the engine's own level-0 tiles, slot 1 gets two more
-            self._slots = [list(st.bufs), [ctx.dense_alloc(st.rows, self.k), ctx.dense_alloc(st.rows, self.k)]]
+            self._slots = [list(st.bufs), [self._tile(st.rows), self._tile(st.rows)]]
             self._slot_i = 0
         s = self._slot_i % 2
         slot = self._slots[s]
@@ -327,15 +354,16 @@ class ArrowEngine:
         return 2.0 * self.total_nnz * self.k
 
     def algorithmic_bytes_per_step(self) -> float:
-        """Per level nnz*8 + (R+1)*4 + U*k*4 + R*k*4 (U = R = active rows), plus the exchanges
-        (forward 2 passes, backward 3 passes over the routed rows) -- the figure a fused
+        """Per level nnz*8 + (R+1)*4 + U*k*e + R*k*e (U = R = active rows, e = bytes per feature element), plus the
+        exchanges (forward 2 passes, backward 3 passes over the routed rows) -- the figure a fused
         implementation still reports against."""
+        e = self.itemsize
         total = 0.0
         for j, st in enumerate(self.levels):
-            total += st.nnz * 8 + (st.rows + 1) * 4 + 2.0 * st.rows * self.k * 4
+            total += st.nnz * 8 + (st.rows + 1) * 4 + 2.0 * st.rows * self.k * e
             if j > 0:
                 m = int(np.count_nonzero(st.to_prev < self.levels[j - 1].rows))
-                total += 5.0 * m * self.k * 4
+                total += 5.0 * m * self.k * e
         return total
 
     def _launch_level_as_in_step(self, j: int, src, dst):
@@ -353,7 +381,7 @@ class ArrowEngine:
         if j > 0 and self.mode == "fused":
             raise ValueError("levels > 0 are timed through step() in fused mode")
         src = st.bufs[st.xi]
-        scratch = self.ctx.dense_alloc(st.rows, self.k)
+        scratch = self._tile(st.rows)
         for _ in range(warmup):
             self._launch_level_as_in_step(j, src, scratch)
         self.ctx.timer_start(5)
@@ -365,14 +393,15 @@ class ArrowEngine:
         return ms
 
     def level_bytes(self, j: int) -> float:
-        """algorithmic bytes of level ``j``'s launch: nnz*8 + (R+1)*4 + R*k*4 (X) + R*k*4 (C), plus -- when the launch
-        carries the epilogue gather-add -- one read of the routed rows of the deeper level's tile (the other two passes
-        of the reference's backward exchange do not exist in this launch)"""
+        """algorithmic bytes of level ``j``'s launch: nnz*8 + (R+1)*4 + R*k*e (X) + R*k*e (C), e = bytes per feature
+        element, plus -- when the launch carries the epilogue gather-add -- one read of the routed rows of the deeper
+        level's tile (the other two passes of the reference's backward exchange do not exist in this launch)"""
         st = self.levels[j]
-        b = st.nnz * 8 + (st.rows + 1) * 4 + 2.0 * st.rows * self.k * 4
+        e = self.itemsize
+        b = st.nnz * 8 + (st.rows + 1) * 4 + 2.0 * st.rows * self.k * e
         if self.mode == "fused" and self.fused_style == "gather" and j + 1 < self.L:
             nxt = self.levels[j + 1]
-            b += float(np.count_nonzero(nxt.to_prev < st.rows)) * self.k * 4
+            b += float(np.count_nonzero(nxt.to_prev < st.rows)) * self.k * e
         return b
 
     def close(self):

@@ -14,7 +14,9 @@
  * arrow_last_error), no exceptions cross the boundary.  The caller owns host memory; the library
  * owns device memory (handles are small non-negative ints, valid for one context).  All work is
  * stream-ordered on the context's stream; arrow_sync() waits for it.  One host thread per context.
- * Dense tiles are row-major fp32 [rows x k]; CSR is fp32 values with int32 indices on the device.
+ * Dense tiles are row-major [rows x k] of fp32 (default) or bf16 (ARROW_DTYPE_BF16, one-GPU launches only); CSR is fp32
+ * values with int32 indices on the device.  Arithmetic is fp32 in both: a kernel widens bf16 inputs to fp32, accumulates
+ * in fp32 and rounds every stored bf16 row once, to nearest even.
  */
 #ifndef ARROW_B200_H
 #define ARROW_B200_H
@@ -28,7 +30,7 @@ extern "C" {
 
 typedef struct arrow_ctx arrow_ctx;
 
-#define ARROW_ABI_VERSION 2
+#define ARROW_ABI_VERSION 3
 
 /* error codes */
 #define ARROW_OK              0
@@ -82,7 +84,8 @@ int  arrow_set_tuning(arrow_ctx *ctx, int long_row_threshold, int long_row_segme
                                         the SM's 228 KB is L1, the landing buffer of the gathers in flight (measurement switch) */
 #define ARROW_OPT_FORCE_PREDICATED 11  /* 1: the tile kernel takes its predicated gather path even when every column is valid (measurement switch) */
 #define ARROW_OPT_TILE_KERNEL     12   /* 1 (default): plain / row-map / accumulate launches with one row per lane group run the round-1 tile
-                                        kernel, 0: the generalised kernel everywhere (A/B switch, profiles/r02_kernel_sweep.md) */
+                                        kernel, 0: the generalised kernel everywhere (A/B switch, profiles/r02_kernel_sweep.md).  fp32
+                                        only: bf16 launches always run the round-1 kernel */
 #define ARROW_OPT_PUSH_INTERLEAVE 13   /* 1 (default): arrow_push_rows walks its destination blocks interleaved (every peer is written to at
                                         every instant); 0: block after block */
 #define ARROW_OPT_BARRIER_TIMEOUT_MS 9 /* arrow_peer_barrier gives up after this long (default 30000) and poisons the context */
@@ -121,12 +124,26 @@ int  arrow_map_invert(arrow_ctx *ctx, int map, int64_t n_out, int *map_out);
 int  arrow_map_d2h(arrow_ctx *ctx, int map, int32_t *host, int64_t n);
 
 /* ---- dense tiles (X_i / C_i / X_0 / C_0 of arrow_slim_mpi.py:354-394, concatenated) ----------- */
-int  arrow_dense_alloc(arrow_ctx *ctx, int64_t rows, int k, int *buf_out);      /* zero filled */
+/* Element types of a dense tile.  Every launch needs all its tiles in one dtype (ARROW_ERR_ARG otherwise).  bf16 tiles
+ * serve the one-GPU launches (arrow_spmm, arrow_spmm_add, arrow_gather_rows, arrow_dense_*); the N-GPU entry points
+ * (arrow_spmm_ex, arrow_push_rows, arrow_reduce_rows, arrow_gather_rows_multi, arrow_ipc_export) refuse them, and
+ * arrow_dense_wrap / arrow_ipc_import make fp32 tiles. */
+#define ARROW_DTYPE_F32  0
+#define ARROW_DTYPE_BF16 1
+int  arrow_dense_alloc(arrow_ctx *ctx, int64_t rows, int k, int *buf_out);      /* zero filled, fp32 */
+int  arrow_dense_alloc_dtype(arrow_ctx *ctx, int64_t rows, int k, int dtype, int *buf_out);   /* zero filled */
+int  arrow_dense_dtype(arrow_ctx *ctx, int buf, int *dtype);
 int  arrow_dense_free(arrow_ctx *ctx, int buf);
-int  arrow_dense_fill(arrow_ctx *ctx, int buf, float value);
+int  arrow_dense_fill(arrow_ctx *ctx, int buf, float value);      /* bf16 tiles: value rounded to nearest even */
+/* fp32 tiles only (a bf16 tile is refused): */
 int  arrow_dense_h2d(arrow_ctx *ctx, int buf, int64_t row0, int64_t rows, const float *host);
 int  arrow_dense_d2h(arrow_ctx *ctx, int buf, int64_t row0, int64_t rows, float *host);
-int  arrow_dense_copy(arrow_ctx *ctx, int dst, int64_t dst_row0, int src, int64_t src_row0, int64_t rows);
+/* Rows in the tile's own dtype (rows x k x 4 or 2 bytes), on copy lane `lane` (ARROW_LANE_*, below; ARROW_LANE_MAIN =
+ * the context's stream).  Stream-ordered like arrow_dense_h2d / d2h: the host memory must stay valid until the lane
+ * has been synchronised. */
+int  arrow_dense_put(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_t rows, const void *host);
+int  arrow_dense_get(arrow_ctx *ctx, int lane, int buf, int64_t row0, int64_t rows, void *host);
+int  arrow_dense_copy(arrow_ctx *ctx, int dst, int64_t dst_row0, int src, int64_t src_row0, int64_t rows);   /* equal dtypes */
 int  arrow_dense_ptr(arrow_ctx *ctx, int buf, void **device_ptr, int64_t *rows, int *k);
 /* Wrap device memory owned by someone else (a torch tensor, an IPC-imported peer tile). */
 int  arrow_dense_wrap(arrow_ctx *ctx, void *device_ptr, int64_t rows, int k, int *buf_out);
