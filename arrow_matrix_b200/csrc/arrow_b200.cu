@@ -139,6 +139,8 @@ struct arrow_ctx {
     bool poisoned = false;            // a peer barrier timed out: later launches are refused (results would be racy)
     float *long_scratch[ARROW_N_LANES] = {};    // [slots][k] partial sums of long-row segments, per lane
     size_t long_scratch_bytes[ARROW_N_LANES] = {};
+    std::vector<float *> retired_scratch;       // replaced long-row scratch a recorded graph may still address: freed
+                                                // with the last graph (arrow_graph_free) or the context
     void *flush_buf = nullptr;
     size_t flush_bytes = 0;
     unsigned int *barrier_epoch = nullptr;        // device: one epoch counter per lane (each lane has its own flag set);
@@ -220,6 +222,12 @@ IdxMap *get_map(arrow_ctx *ctx, int h) {
     } while (0)
 
 inline int ceil_div_i64(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
+
+bool graphs_live(const arrow_ctx *ctx) {
+    for (auto g : ctx->graphs)
+        if (g) return true;
+    return false;
+}
 
 // frees whatever device arrays the block owns (cudaFree waits for the device, so no launch can still read them)
 void csr_release(Csr &c) {
@@ -1890,6 +1898,7 @@ void arrow_ctx_destroy(arrow_ctx *ctx) {
     }
     for (int l = 0; l < ARROW_N_LANES; ++l)
         if (ctx->long_scratch[l]) cudaFree(ctx->long_scratch[l]);
+    for (float *p : ctx->retired_scratch) cudaFree(p);
     for (auto &pt : ctx->ptrtabs)
         if (pt.live) cudaFree(pt.p);
     for (auto g : ctx->graphs)
@@ -2652,7 +2661,12 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
         if (need > ctx->long_scratch_bytes[lane]) {
             if (ctx->capturing) return fail(ctx, ARROW_ERR_UNSUPPORTED, "long-row scratch would grow during graph capture: run the step once first");
             CUDA_TRY(ctx, cudaStreamSynchronize(stream));
-            if (ctx->long_scratch[lane]) cudaFree(ctx->long_scratch[lane]);
+            // a graph recorded earlier replays with the pointer it captured: while one is live the old buffer is retired,
+            // not freed, so that a replay after this growth still reads and writes memory it owns
+            if (ctx->long_scratch[lane]) {
+                if (graphs_live(ctx)) ctx->retired_scratch.push_back(ctx->long_scratch[lane]);
+                else cudaFree(ctx->long_scratch[lane]);
+            }
             ctx->long_scratch[lane] = nullptr;
             ctx->long_scratch_bytes[lane] = 0;
             CUDA_TRY(ctx, cudaMalloc(&ctx->long_scratch[lane], need));
@@ -3226,6 +3240,10 @@ int arrow_graph_free(arrow_ctx *ctx, int graph) {
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     cudaGraphExecDestroy(ctx->graphs[graph]);
     ctx->graphs[graph] = nullptr;
+    if (!graphs_live(ctx)) {                                  // no replay can address a retired scratch buffer any more
+        for (float *p : ctx->retired_scratch) cudaFree(p);
+        ctx->retired_scratch.clear();
+    }
     return ARROW_OK;
 }
 
