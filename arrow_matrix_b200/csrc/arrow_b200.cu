@@ -8,7 +8,8 @@
 //   remapped columns    arrow_dec_mpi.py:526,544  (`feature_tile()[perm]` + `C_i[perm] = recvbuf`)
 //   k_gather_rows*      the same two exchanges as standalone (un-fused / cross-GPU) steps
 //
-// Layout: CSR = int32 indptr (rebased to 0) / int32 indices / fp32 values; dense tiles row-major fp32 or bf16 (one-GPU
+// Layout: CSR = 4-byte row pointer holding the low 32 bits of 64-bit offsets (rebased to 0; tiles, long-row tasks and
+// 64-row anchors carry the 64-bit bases) / int32 indices / fp32 values; dense tiles row-major fp32 or bf16 (one-GPU
 // launches; fp32 arithmetic, each stored bf16 row rounded once to nearest even).
 // All kernels are HBM/L2-bandwidth bound gathers (about 2 FLOP/B): no tensor cores on purpose.
 #include "../../include/arrow_b200.h"
@@ -52,15 +53,20 @@ struct DenseBuf {
 };
 
 struct LongTask {      // one segment of a long row
+    long long begin;   // nnz offsets (rebased, 64-bit)
+    long long end;
     int row;
-    int begin;         // nnz offsets (rebased)
-    int end;
     int slot;          // partial-sum slot
 };
 
+// Rows per anchor of the per-row kernels: the 64-bit offset of row r is anchors[r / ROW_GROUP] plus the 32-bit wrapping
+// difference of the row pointer's low words, exact while one group spans fewer than 2^32 entries (checked at upload).
+constexpr int ROW_GROUP_SHIFT = 6;
+constexpr int ROW_GROUP = 1 << ROW_GROUP_SHIFT;
+
 struct Csr {
     int64_t n_rows = 0, n_cols = 0, nnz = 0;
-    int *indptr = nullptr;
+    int *indptr = nullptr;            // low 32 bits of each row's 64-bit first entry
     int *indices = nullptr;
     float *vals = nullptr;
     bool owns_indptr = false, owns_indices = false, owns_vals = false;
@@ -74,10 +80,14 @@ struct Csr {
     int *long_first = nullptr;        // device: first slot of each long row (n_long_rows+1)
     bool owns_long = false;
     int long_threshold = 0;
-    // row tiles for the CSR-streaming kernel: {row_begin, row_end, nnz_begin, nnz_end}
+    long long *anchors = nullptr;     // device: 64-bit first entry of every ROW_GROUP-th row (owned with the long rows)
+    // row tiles for the CSR-streaming kernel: {row_begin, row_end, low 32 bits of nnz_begin, of nnz_end}, and the
+    // tile's 64-bit nnz_begin in a parallel array
     int4 *tiles = nullptr;
+    long long *tile_base = nullptr;
     int n_tiles = 0;
     int4 *tiles_big = nullptr;        // TILE_ROWS_BIG / TILE_NNZ_BIG variant for narrow feature tiles
+    long long *tile_base_big = nullptr;
     int n_tiles_big = 0;
     int parent = -1;                  // handle of the block whose indptr / values / tiles this one shares (remapped copy)
     int children = 0;                 // live remapped copies that share this block's arrays
@@ -240,6 +250,9 @@ void csr_release(Csr &c) {
         cudaFree(c.long_first);
         cudaFree(c.tiles);
         cudaFree(c.tiles_big);
+        cudaFree(c.tile_base);
+        cudaFree(c.tile_base_big);
+        cudaFree(c.anchors);
     }
     c = Csr();
 }
@@ -324,7 +337,8 @@ template <typename T>
 constexpr bool is_bf16() { return std::is_same<T, bf16>::value; }
 
 struct SpmmArgs {
-    const int *__restrict__ indptr;
+    const int *__restrict__ indptr;   // low 32 bits of the 64-bit row offsets
+    const long long *__restrict__ anchors;   // 64-bit offset of every ROW_GROUP-th row (per-row kernels)
     const int *__restrict__ indices;
     const float *__restrict__ vals;
     const float *__restrict__ X;      // dense tiles (X, C, X2, add_src) hold the launch's element type T (Elt<T>)
@@ -340,6 +354,17 @@ struct SpmmArgs {
     int x_split;
     float *const *__restrict__ out_ptr;  // optional destination pointer per row (nullptr entry = row dropped); overrides C / rowmap
 };
+
+// a - b of two row-pointer low words: exact for any two offsets less than 2^32 apart (no signed overflow)
+__device__ __forceinline__ int wdiff(int a, int b) { return (int)((unsigned)a - (unsigned)b); }
+
+// 64-bit first entry and length of `row` (per-row kernels)
+__device__ __forceinline__ long long row_begin(const SpmmArgs &a, long long row, long long &len) {
+    const long long anchor = __ldg(a.anchors + (row >> ROW_GROUP_SHIFT));
+    const int lo = __ldg(a.indptr + row);
+    len = (unsigned)wdiff(__ldg(a.indptr + row + 1), lo);
+    return anchor + (unsigned)wdiff(lo, (int)anchor);
+}
 
 // ------------------------------------------------------------------------------------------------
 // variant 0: a group of G lanes owns one row; every lane of the group reads the same index/value
@@ -362,9 +387,10 @@ __global__ void __launch_bounds__(256, 4) k_spmm_direct(SpmmArgs a) {
     const int k4 = a.k4;
 
     for (long long row = warp_id * RPW + gi; row < a.n_rows; row += warps_total * RPW) {
-        const int s = __ldg(a.indptr + row);
-        const int e = __ldg(a.indptr + row + 1);
-        if (e - s > a.long_threshold) continue;
+        long long len;
+        const long long s = row_begin(a, row, len);
+        if (len > a.long_threshold) continue;
+        const long long e = s + len;
         long long orow = row;
         if (ROWMAP) {
             orow = __ldg(a.rowmap + row);
@@ -374,7 +400,7 @@ __global__ void __launch_bounds__(256, 4) k_spmm_direct(SpmmArgs a) {
 #pragma unroll
         for (int i = 0; i < VPL; ++i) acc[i] = f4_zero();
 
-        for (int p = s; p < e; p += UNROLL) {
+        for (long long p = s; p < e; p += UNROLL) {
             int c[UNROLL];
             float v[UNROLL];
 #pragma unroll
@@ -434,16 +460,17 @@ __global__ void __launch_bounds__(256, 4) k_spmm_shfl(SpmmArgs a) {
     // warp-uniform trip count: every lane of the warp runs the same number of row iterations
     for (long long row0 = warp_id * RPW; row0 < a.n_rows; row0 += warps_total * RPW) {
         const long long row = row0 + gi;
-        int s = 0, e = 0;
+        long long s = 0;
+        int len = 0;
         long long orow = -1;
         if (row < a.n_rows) {
-            s = __ldg(a.indptr + row);
-            e = __ldg(a.indptr + row + 1);
+            long long n;
+            s = row_begin(a, row, n);
             orow = row;
             if (ROWMAP) orow = __ldg(a.rowmap + row);
-            if (e - s > a.long_threshold || orow < 0) { e = s; orow = -1; }
+            if (n > a.long_threshold || orow < 0) orow = -1;
+            else len = (int)n;
         }
-        const int len = e - s;
         const int maxlen = __reduce_max_sync(0xffffffffu, len);
         float4 acc[VPL];
 #pragma unroll
@@ -593,7 +620,7 @@ constexpr int TMA_STAGES = 2;
 struct TmaItem {
     long long row;     // -1: end of stream
     long long orow;
-    int p0;            // first nnz of this chunk
+    long long p0;      // first nnz of this chunk
     int cnt;           // nnz in this chunk
     int last;          // chunk closes its row
     int myc;           // this lane's column (lane < cnt), -1 otherwise
@@ -623,21 +650,21 @@ __global__ void __launch_bounds__(TMA_WARPS * 32) k_spmm_tma(SpmmArgs a) {
 
     // work-item iterator (all lanes hold identical copies)
     long long it_row = warp_id - warps_total;
-    int it_p = 0, it_e = 0;
+    long long it_p = 0, it_e = 0;
     long long it_orow = -1;
     auto next_item = [&](TmaItem &t) {
         while (it_p >= it_e) {                       // advance to the next non-empty, non-long, routed row
             it_row += warps_total;
             if (it_row >= a.n_rows) { t.row = -1; t.cnt = 0; t.myc = -1; t.myv = 0.f; t.last = 0; return; }
-            const int s = __ldg(a.indptr + it_row);
-            const int e = __ldg(a.indptr + it_row + 1);
+            long long len;
+            const long long s = row_begin(a, it_row, len);
             long long orow = it_row;
             if (ROWMAP) orow = __ldg(a.rowmap + it_row);
-            if (orow < 0 || e - s > a.long_threshold) continue;
+            if (orow < 0 || len > a.long_threshold) continue;
             it_orow = orow;
             it_p = s;
-            it_e = e;
-            if (s == e) {                            // empty row still has to store zeros / keep C
+            it_e = s + len;
+            if (len == 0) {                          // empty row still has to store zeros / keep C
                 t.row = it_row; t.orow = orow; t.p0 = s; t.cnt = 0; t.last = 1; t.myc = -1; t.myv = 0.f;
                 return;
             }
@@ -645,7 +672,7 @@ __global__ void __launch_bounds__(TMA_WARPS * 32) k_spmm_tma(SpmmArgs a) {
         t.row = it_row;
         t.orow = it_orow;
         t.p0 = it_p;
-        t.cnt = min(TMA_SLOTS, it_e - it_p);
+        t.cnt = (int)min((long long)TMA_SLOTS, it_e - it_p);
         it_p += t.cnt;
         t.last = (it_p >= it_e);
         t.myc = -1;
@@ -741,6 +768,7 @@ constexpr int OUT_ROWPTR = 2;       // *(out_ptr[r])          (device pointer pe
 struct TileArgs {
     SpmmArgs a;
     const int4 *__restrict__ tiles;
+    const long long *__restrict__ tile_base;   // 64-bit nnz_begin of each tile: the source of its bulk copies
     int n_tiles;
     int skip;            // indices may hold -1
     int *ticket;         // dynamic tile scheduler: [0] next tile, [1] CTAs that finished (the last one re-arms both)
@@ -791,9 +819,9 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
     auto prefetch = [&](int tile, int st) {
         const int4 d = __ldg(t.tiles + tile);
         const int rb4 = d.x & ~3;
-        const int a0 = d.z & ~3;
+        const long long a0 = __ldg(t.tile_base + tile) & ~3LL;
         const uint32_t ptr_bytes = (uint32_t)(((d.y - rb4 + 1) + 3) & ~3) * 4u;
-        const uint32_t nnz_bytes = (uint32_t)(((d.w - a0) + 3) & ~3) * 4u;
+        const uint32_t nnz_bytes = (uint32_t)((wdiff(d.w, d.z & ~3) + 3) & ~3) * 4u;
         int *sp = stage_base + (size_t)st * TILE_STAGE_WORDS;
         mbar_expect_tx(&bars[st], ptr_bytes + 2u * nnz_bytes);
         bulk_g2s_hint(sp, a.indptr + rb4, ptr_bytes, &bars[st], pol_stream);
@@ -823,14 +851,14 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
         else         { mbar_wait(&bars[1], parity1); parity1 ^= 1u; }
         const int *sp = stage_base + (size_t)st * TILE_STAGE_WORDS;
         const int *s_ptr = sp + (d.x - (d.x & ~3));
-        const int a0 = d.z & ~3;
-        const int *s_idx = sp + TILE_PTR_WORDS - a0;                    // index with global nnz offsets
-        const float *s_val = reinterpret_cast<const float *>(sp + TILE_PTR_WORDS + TILE_NNZ_WORDS) - a0;
+        const int a0 = d.z & ~3;                                        // low word of the slice's first entry
+        const int *s_idx = sp + TILE_PTR_WORDS;                         // index with tile-local offsets
+        const float *s_val = reinterpret_cast<const float *>(sp + TILE_PTR_WORDS + TILE_NNZ_WORDS);
         const int n_rows_tile = d.y - d.x;
 
         for (int lr = warp * RPW + gi; lr < n_rows_tile; lr += (TILE_THREADS / 32) * RPW) {
-            const int s = s_ptr[lr];
-            const int e = s_ptr[lr + 1];
+            const int s = wdiff(s_ptr[lr], a0);
+            const int e = wdiff(s_ptr[lr + 1], a0);
             if (e - s > a.long_threshold) continue;
             const long long row = (long long)d.x + lr;
             long long orow = row;
@@ -843,7 +871,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles_v1(TileArgs t) {
                 // indices are already in shared memory); hides DRAM latency of first-touch / scattered rows
                 const int nlr = lr + (TILE_THREADS / 32) * RPW;
                 if (nlr < n_rows_tile) {
-                    const int ns = s_ptr[nlr], ne = s_ptr[nlr + 1];
+                    const int ns = wdiff(s_ptr[nlr], a0), ne = wdiff(s_ptr[nlr + 1], a0);
                     if (ne - ns <= a.long_threshold) {
                         const int lines = (a.k * 4 + 127) >> 7;
                         for (int q = ns + gl; q < ne; q += G) {
@@ -982,9 +1010,9 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
     auto issue_csr = [&](int tile, int st) {
         const int4 d = __ldg(t.tiles + tile);
         const int rb4 = d.x & ~3;
-        const int a0 = d.z & ~3;
+        const long long a0 = __ldg(t.tile_base + tile) & ~3LL;
         const uint32_t ptr_bytes = (uint32_t)(((d.y - rb4 + 1) + 3) & ~3) * 4u;
-        const uint32_t nnz_bytes = (uint32_t)(((d.w - a0) + 3) & ~3) * 4u;
+        const uint32_t nnz_bytes = (uint32_t)((wdiff(d.w, d.z & ~3) + 3) & ~3) * 4u;
         int *sp = stage_base + (size_t)st * TILE_STAGE_WORDS;
         mbar_expect_tx(&bars[st], ptr_bytes + 2u * nnz_bytes);
         bulk_g2s_hint(sp, a.indptr + rb4, ptr_bytes, &bars[st], pol_stream);
@@ -1019,9 +1047,9 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
         phase ^= (1u << st);
         const int *sp = stage_base + (size_t)st * TILE_STAGE_WORDS;
         const int *s_ptr = sp + (d.x - (d.x & ~3));
-        const int a0 = d.z & ~3;
-        const int *s_idx = sp + TILE_PTR_WORDS - a0;                    // index with global nnz offsets
-        const float *s_val = reinterpret_cast<const float *>(sp + TILE_PTR_WORDS + TILE_NNZ_WORDS) - a0;
+        const int a0 = d.z & ~3;                                        // low word of the slice's first entry
+        const int *s_idx = sp + TILE_PTR_WORDS;                         // index with tile-local offsets
+        const float *s_val = reinterpret_cast<const float *>(sp + TILE_PTR_WORDS + TILE_NNZ_WORDS);
         const int n_rows_tile = d.y - d.x;
 
         if (t.prefetch) {
@@ -1029,7 +1057,7 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
             // registers, no LSU wavefronts).  Measured in round 2 (profiles/r02_kernel_sweep.md): a LOSS at every k -- the
             // request rate of the unit, not DRAM latency, becomes the bound.  Off by default; kept as the A/B switch.
             const uint32_t row_bytes = (uint32_t)a.k * (uint32_t)sizeof(T);
-            for (int q = d.z + (int)threadIdx.x; q < d.w; q += TILE_THREADS) {
+            for (int q = wdiff(d.z, a0) + (int)threadIdx.x; q < wdiff(d.w, a0); q += TILE_THREADS) {
                 const int cq = s_idx[q];
                 if (cq >= 0) bulk_prefetch_l2(xrow(cq) - gl, row_bytes);
             }
@@ -1049,8 +1077,8 @@ __global__ void __launch_bounds__(TILE_THREADS, 4) k_spmm_tiles(TileArgs t) {
                 p[r] = e[r] = 0;
                 cr[r] = nullptr;
                 if (live[r]) {
-                    p[r] = s_ptr[lr];
-                    e[r] = s_ptr[lr + 1];
+                    p[r] = wdiff(s_ptr[lr], a0);
+                    e[r] = wdiff(s_ptr[lr + 1], a0);
                     if (e[r] - p[r] > a.long_threshold) { live[r] = false; e[r] = p[r]; }
                 }
                 const long long row = (long long)d.x + lr;
@@ -1233,9 +1261,10 @@ __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
     const long long warps_total = (long long)gridDim.x * (blockDim.x >> 5);
     const long long warp_id = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     for (long long row = warp_id; row < a.n_rows; row += warps_total) {
-        const int s = __ldg(a.indptr + row);
-        const int e = __ldg(a.indptr + row + 1);
-        if (e - s > a.long_threshold) continue;
+        long long len;
+        const long long s = row_begin(a, row, len);
+        if (len > a.long_threshold) continue;
+        const long long e = s + len;
         long long orow = row;
         if (ROWMAP) {
             orow = __ldg(a.rowmap + row);
@@ -1248,7 +1277,7 @@ __global__ void __launch_bounds__(256) k_spmm_generic(SpmmArgs a) {
         }
         for (int c0 = 0; c0 < a.k; c0 += 128) {
             float acc[4] = {0.f, 0.f, 0.f, 0.f};
-            for (int p = s; p < e; ++p) {
+            for (long long p = s; p < e; ++p) {
                 const int c = __ldg(a.indices + p);
                 const float v = __ldg(a.vals + p);
                 if (c < 0) continue;
@@ -1298,7 +1327,7 @@ __global__ void __launch_bounds__(256) k_spmm_long_partial(LongArgs a) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
     for (int c0 = 0; c0 < a.k; c0 += 128) {
         float acc[4] = {0.f, 0.f, 0.f, 0.f};
-        for (int p = t.begin + warp; p < t.end; p += nwarps) {
+        for (long long p = t.begin + warp; p < t.end; p += nwarps) {
             const int c = __ldg(a.indices + p);
             const float v = __ldg(a.vals + p);
             if (c < 0) continue;
@@ -1784,7 +1813,7 @@ int launch_tiles(arrow_ctx *ctx, TileArgs &t, const Csr *A, const TileLaunch &L)
     int g = 1;
     while (g < lanes) g <<= 1;
     const bool big = (k4 <= 8) && ctx->big_tiles && A->n_tiles_big > 0;     // rows of <= 128 bytes (fp32 k <= 32, bf16 k <= 64)
-    if (big) { t.tiles = A->tiles_big; t.n_tiles = A->n_tiles_big; }
+    if (big) { t.tiles = A->tiles_big; t.tile_base = A->tile_base_big; t.n_tiles = A->n_tiles_big; }
     // measured at 10M rows (profiles/r02_kernel_sweep.md): pairs win at k = 32 (+3.5 %), lose at k = 16 (-10 %)
     int rpg = L.rpg_req ? L.rpg_req : (ctx->rows_per_group ? ctx->rows_per_group : (vpl == 2 ? 2 : 1));
     if (!big || rpg != 2) rpg = 1;                                           // pairs need >= 2 passes per tile
@@ -1972,53 +2001,66 @@ int arrow_set_option(arrow_ctx *ctx, int option, int value) {
 }
 
 // ---- sparse -------------------------------------------------------------------------------------
-static int build_long_rows(arrow_ctx *ctx, Csr &c, const std::vector<int> &h_indptr) {
+inline int low_word(int64_t v) { return (int)(uint32_t)(uint64_t)v; }
+
+static int build_long_rows(arrow_ctx *ctx, Csr &c, const std::vector<int64_t> &h_indptr) {
     // host pass over the (rebased) row pointer: rows above the threshold become segment tasks
     std::vector<LongTask> tasks;
     std::vector<int> rows, first;
     int64_t mx = 0;
     const int thr = ctx->long_threshold, seg = ctx->long_segment;
     for (int64_t r = 0; r < c.n_rows; ++r) {
-        const int len = h_indptr[r + 1] - h_indptr[r];
+        const int64_t len = h_indptr[r + 1] - h_indptr[r];
         mx = std::max<int64_t>(mx, len);
         if (len > thr) {
             rows.push_back((int)r);
             first.push_back((int)tasks.size());
-            for (int b = h_indptr[r]; b < h_indptr[r + 1]; b += seg)
-                tasks.push_back(LongTask{(int)r, b, std::min(b + seg, h_indptr[r + 1]), (int)tasks.size()});
+            for (int64_t b = h_indptr[r]; b < h_indptr[r + 1]; b += seg)
+                tasks.push_back(LongTask{b, std::min<int64_t>(b + seg, h_indptr[r + 1]), (int)r, (int)tasks.size()});
         }
     }
     first.push_back((int)tasks.size());
     // row tiles for k_spmm_tiles: contiguous rows, <= rows_cap rows and <= nnz_cap entries, cut around long rows
-    auto build_tiles = [&](int rows_cap, int nnz_cap, int4 **out, int *n_out) -> int {
+    auto build_tiles = [&](int rows_cap, int nnz_cap, int4 **out, long long **base_out, int *n_out) -> int {
         std::vector<int4> tiles;
+        std::vector<long long> base;
         int64_t r = 0;
         while (r < c.n_rows) {
-            const int len0 = h_indptr[r + 1] - h_indptr[r];
+            const int64_t len0 = h_indptr[r + 1] - h_indptr[r];
             if (len0 > thr) { ++r; continue; }                     // long rows are not tiled
             int64_t e = r;
             while (e < c.n_rows && e - r < rows_cap) {
-                const int len = h_indptr[e + 1] - h_indptr[e];
+                const int64_t len = h_indptr[e + 1] - h_indptr[e];
                 if (len > thr) break;
                 if (h_indptr[e + 1] - h_indptr[r] > nnz_cap - 4 && e > r) break;
                 ++e;
             }
             if (e == r) ++e;                                       // a single row always fits: thr <= TILE_NNZ - 8
-            tiles.push_back(make_int4((int)r, (int)e, h_indptr[r], h_indptr[e]));
+            tiles.push_back(make_int4((int)r, (int)e, low_word(h_indptr[r]), low_word(h_indptr[e])));
+            base.push_back(h_indptr[r]);
             r = e;
         }
         *n_out = (int)tiles.size();
         if (!tiles.empty()) {
             CUDA_TRY(ctx, cudaMalloc(out, tiles.size() * sizeof(int4)));
             CUDA_TRY(ctx, cudaMemcpy(*out, tiles.data(), tiles.size() * sizeof(int4), cudaMemcpyHostToDevice));
+            CUDA_TRY(ctx, cudaMalloc(base_out, base.size() * sizeof(long long)));
+            CUDA_TRY(ctx, cudaMemcpy(*base_out, base.data(), base.size() * sizeof(long long), cudaMemcpyHostToDevice));
         }
         return ARROW_OK;
     };
     {
-        int rc = build_tiles(TILE_ROWS, TILE_NNZ, &c.tiles, &c.n_tiles);
+        int rc = build_tiles(TILE_ROWS, TILE_NNZ, &c.tiles, &c.tile_base, &c.n_tiles);
         if (rc != ARROW_OK) return rc;
-        rc = build_tiles(TILE_ROWS_BIG, TILE_NNZ_BIG, &c.tiles_big, &c.n_tiles_big);
+        rc = build_tiles(TILE_ROWS_BIG, TILE_NNZ_BIG, &c.tiles_big, &c.tile_base_big, &c.n_tiles_big);
         if (rc != ARROW_OK) return rc;
+    }
+    {
+        std::vector<long long> anchors((size_t)((c.n_rows + ROW_GROUP - 1) >> ROW_GROUP_SHIFT) + 1);
+        for (size_t g = 0; g < anchors.size(); ++g)
+            anchors[g] = h_indptr[std::min<int64_t>((int64_t)g << ROW_GROUP_SHIFT, c.n_rows)];
+        CUDA_TRY(ctx, cudaMalloc(&c.anchors, anchors.size() * sizeof(long long)));
+        CUDA_TRY(ctx, cudaMemcpy(c.anchors, anchors.data(), anchors.size() * sizeof(long long), cudaMemcpyHostToDevice));
     }
     c.max_row_nnz = mx;
     c.long_threshold = thr;
@@ -2037,15 +2079,17 @@ static int build_long_rows(arrow_ctx *ctx, Csr &c, const std::vector<int> &h_ind
 }
 
 // device side of arrow_csr_upload; on failure the caller releases whatever `c` already owns
-static int csr_fill(arrow_ctx *ctx, Csr &c, int64_t n_rows, int64_t n_cols, int64_t nnz, const std::vector<int> &h_indptr,
+static int csr_fill(arrow_ctx *ctx, Csr &c, int64_t n_rows, int64_t n_cols, int64_t nnz, const std::vector<int64_t> &h_indptr,
                     const void *indices, int indices_bytes, const float *data) {
     c.n_rows = n_rows;
     c.n_cols = n_cols;
     c.nnz = nnz;
     c.owns_indptr = c.owns_indices = c.owns_vals = c.owns_long = true;     // every array below belongs to this block
+    std::vector<int> h_low((size_t)n_rows + 1);              // the device row pointer: low 32 bits of every offset
+    for (size_t r = 0; r < h_low.size(); ++r) h_low[r] = low_word(h_indptr[r]);
     CUDA_TRY(ctx, cudaMalloc(&c.indptr, ((size_t)n_rows + 1 + 8) * sizeof(int)));
     CUDA_TRY(ctx, cudaMemsetAsync(c.indptr, 0, ((size_t)n_rows + 1 + 8) * sizeof(int), ctx->stream));
-    CUDA_TRY(ctx, cudaMemcpyAsync(c.indptr, h_indptr.data(), ((size_t)n_rows + 1) * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(ctx, cudaMemcpyAsync(c.indptr, h_low.data(), ((size_t)n_rows + 1) * sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
     const size_t nz = (size_t)nnz + 8;                       // slack: bulk copies round up to 16 bytes
     CUDA_TRY(ctx, cudaMalloc(&c.indices, nz * sizeof(int)));
     CUDA_TRY(ctx, cudaMalloc(&c.vals, nz * sizeof(float)));
@@ -2059,10 +2103,16 @@ static int csr_fill(arrow_ctx *ctx, Csr &c, int64_t n_rows, int64_t n_cols, int6
         if (indices_bytes == 4) {
             CUDA_TRY(ctx, cudaMemcpyAsync(c.indices, indices, (size_t)nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
         } else {
-            CUDA_TRY(ctx, cudaMalloc(&wide.p, (size_t)nnz * 8));
-            CUDA_TRY(ctx, cudaMemcpyAsync(wide.p, indices, (size_t)nnz * 8, cudaMemcpyHostToDevice, ctx->stream));
-            k_to_i32<long long><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>((const long long *)wide.p, c.indices, nnz, 0, (int *)bad.p);
-            ctx->launches++;
+            // 64-bit columns are narrowed through a bounded staging buffer: a block of billions of entries needs no
+            // second copy of its index stream at twice the width
+            const int64_t chunk = std::min<int64_t>(nnz, (int64_t)1 << 26);
+            CUDA_TRY(ctx, cudaMalloc(&wide.p, (size_t)chunk * 8));
+            for (int64_t o = 0; o < nnz; o += chunk) {
+                const int64_t n = std::min(chunk, nnz - o);
+                CUDA_TRY(ctx, cudaMemcpyAsync(wide.p, (const int64_t *)indices + o, (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+                k_to_i32<long long><<<ctx->sm_count * 8, 256, 0, ctx->stream>>>((const long long *)wide.p, c.indices + o, n, 0, (int *)bad.p);
+                ctx->launches++;
+            }
         }
         // a column outside [0, n_cols) would read outside the X tile: reject the block instead
         k_check_cols<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(c.indices, nnz, n_cols, (int *)bad.p);
@@ -2090,11 +2140,11 @@ int arrow_csr_upload(arrow_ctx *ctx, int64_t n_rows, int64_t n_cols, int64_t nnz
     if (n_rows < 0 || n_cols < 0 || nnz < 0) return fail(ctx, ARROW_ERR_ARG, "negative size");
     if ((indptr_bytes != 4 && indptr_bytes != 8) || (indices_bytes != 4 && indices_bytes != 8))
         return fail(ctx, ARROW_ERR_ARG, "index width must be 4 or 8 bytes");
-    if (nnz > 2147483647LL || n_rows >= 2147483647LL || n_cols > 2147483647LL)
-        return fail(ctx, ARROW_ERR_RANGE, "block exceeds the int32 device layout (rows=%lld cols=%lld nnz=%lld); shard it",
-                    (long long)n_rows, (long long)n_cols, (long long)nnz);
+    if (n_rows >= 2147483647LL || n_cols > 2147483647LL)
+        return fail(ctx, ARROW_ERR_RANGE, "rows / columns exceed the int32 device layout (rows=%lld cols=%lld); shard it",
+                    (long long)n_rows, (long long)n_cols);
     // host view of the row pointer, rebased
-    std::vector<int> h_indptr((size_t)n_rows + 1);
+    std::vector<int64_t> h_indptr((size_t)n_rows + 1);
     int64_t base = 0;
     if (indptr_bytes == 8) {
         const int64_t *ip = (const int64_t *)indptr;
@@ -2103,7 +2153,7 @@ int arrow_csr_upload(arrow_ctx *ctx, int64_t n_rows, int64_t n_cols, int64_t nnz
             const int64_t v = ip[r] - base;
             if (v < 0 || v > nnz || (r > 0 && v < h_indptr[r - 1]))
                 return fail(ctx, ARROW_ERR_ARG, "indptr is not a non-decreasing sequence inside [0, nnz] at row %lld", (long long)r);
-            h_indptr[r] = (int)v;
+            h_indptr[r] = v;
         }
     } else {
         const int32_t *ip = (const int32_t *)indptr;
@@ -2112,11 +2162,19 @@ int arrow_csr_upload(arrow_ctx *ctx, int64_t n_rows, int64_t n_cols, int64_t nnz
             const int64_t v = (int64_t)ip[r] - base;
             if (v < 0 || v > nnz || (r > 0 && v < h_indptr[r - 1]))
                 return fail(ctx, ARROW_ERR_ARG, "indptr is not a non-decreasing sequence inside [0, nnz] at row %lld", (long long)r);
-            h_indptr[r] = (int)v;
+            h_indptr[r] = v;
         }
     }
     if (h_indptr[n_rows] != nnz)
-        return fail(ctx, ARROW_ERR_ARG, "indptr[n_rows]-indptr[0] = %d but nnz = %lld", h_indptr[n_rows], (long long)nnz);
+        return fail(ctx, ARROW_ERR_ARG, "indptr[n_rows]-indptr[0] = %lld but nnz = %lld", (long long)h_indptr[n_rows], (long long)nnz);
+    // the per-row kernels find a row's 64-bit offset from the first row of its group of ROW_GROUP rows and a 32-bit
+    // difference: no group may span 2^32 entries (rows averaging 2^26 entries)
+    for (int64_t g = 0; g < n_rows; g += ROW_GROUP) {
+        const int64_t span = h_indptr[std::min<int64_t>(g + ROW_GROUP, n_rows)] - h_indptr[g];
+        if (span > 0xffffffffLL)
+            return fail(ctx, ARROW_ERR_RANGE, "rows %lld..%lld hold %lld entries; a group of %d rows must hold fewer than 2^32",
+                        (long long)g, (long long)std::min<int64_t>(g + ROW_GROUP, n_rows) - 1, (long long)span, ROW_GROUP);
+    }
 
     Csr c;
     const int rc = csr_fill(ctx, c, n_rows, n_cols, nnz, h_indptr, indices, indices_bytes, data);
@@ -2562,6 +2620,7 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
     cudaStream_t stream = cur_stream(ctx);
     SpmmArgs a;
     a.indptr = A->indptr;
+    a.anchors = A->anchors;
     a.indices = A->indices;
     a.vals = A->vals;
     a.X = X->p;
@@ -2626,6 +2685,7 @@ static int spmm_impl(arrow_ctx *ctx, const SpmmCall &q) {
             TileArgs t;
             t.a = a;
             t.tiles = A->tiles;
+            t.tile_base = A->tile_base;
             t.n_tiles = A->n_tiles;
             t.skip = (A->may_skip || ctx->force_skip_path) ? 1 : 0;
             t.ticket = ctx->tile_ticket + 2 * lane;

@@ -15,7 +15,8 @@
  * owns device memory (handles are small non-negative ints, valid for one context).  All work is
  * stream-ordered on the context's stream; arrow_sync() waits for it.  One host thread per context.
  * Dense tiles are row-major [rows x k] of fp32 (default) or bf16 (ARROW_DTYPE_BF16, one-GPU launches only); CSR is fp32
- * values with int32 indices on the device.  Arithmetic is fp32 in both: a kernel widens bf16 inputs to fp32, accumulates
+ * values with int32 column indices on the device and 64-bit non-zero offsets (rows and columns < 2^31, non-zeros bounded
+ * by device memory).  Arithmetic is fp32 in both: a kernel widens bf16 inputs to fp32, accumulates
  * in fp32 and rounds every stored bf16 row once, to nearest even.
  */
 #ifndef ARROW_B200_H
@@ -37,7 +38,7 @@ typedef struct arrow_ctx arrow_ctx;
 #define ARROW_ERR_CUDA       -1
 #define ARROW_ERR_ARG        -2
 #define ARROW_ERR_HANDLE     -3
-#define ARROW_ERR_RANGE      -4   /* index / size exceeds the int32 device layout */
+#define ARROW_ERR_RANGE      -4   /* index / size exceeds the device layout (rows, columns, map entries < 2^31) */
 #define ARROW_ERR_NOMEM      -5
 #define ARROW_ERR_UNSUPPORTED -6
 
@@ -95,9 +96,11 @@ int  arrow_set_option(arrow_ctx *ctx, int option, int value);
 /* indptr has n_rows+1 entries of indptr_bytes (4 or 8) each and may start at any base value
  * (a row slice of a bigger file); indices/data point at the entry indptr[0] refers to.
  * data == NULL means all ones (missing _data.npy, graphio.py:292-298).
+ * nnz may exceed 2^31 - 1 (any size that fits in device memory).
  * Rejected with ARROW_ERR_ARG / ARROW_ERR_RANGE (nothing stays allocated): a row pointer that is not a
- * non-decreasing sequence spanning exactly nnz entries, a column index outside [0, n_cols), a block beyond the
- * int32 device layout. */
+ * non-decreasing sequence spanning exactly nnz entries, a column index outside [0, n_cols), n_rows >= 2^31 - 1 or
+ * n_cols >= 2^31 (ARROW_ERR_RANGE before any host array is read), 64 consecutive rows spanning 2^32 or more entries
+ * (ARROW_ERR_RANGE). */
 int  arrow_csr_upload(arrow_ctx *ctx, int64_t n_rows, int64_t n_cols, int64_t nnz,
                       const void *indptr, int indptr_bytes,
                       const void *indices, int indices_bytes,
